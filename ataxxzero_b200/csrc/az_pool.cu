@@ -159,8 +159,9 @@ int launch_tree(az_pool *pool, Group &grp, bool consume = true)
     grp.dev.tick_slot = grp.slot;
     grp.dev.tick_id++;
     aztree_launch_tick(grp.dev, s);
-    pool->launches++;
-    pool->ctx->launches++;
+    const int kernels = grp.dev.cache_tag ? 1 : 2;        // + k_order_requests
+    pool->launches += kernels;
+    pool->ctx->launches += kernels;
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;
 }
@@ -338,7 +339,7 @@ int drain_finished(az_pool *pool, Group &grp, FILE *out, int64_t *games_written,
 void free_group(Group &grp)
 {
     PoolDev &D = grp.dev;
-    void *ptrs[] = {D.nodes, D.games, D.path, D.gstack, D.req_pos, D.req_game, D.req_count, D.logits, D.values, D.cache_tag,
+    void *ptrs[] = {D.nodes, D.games, D.path, D.gstack, D.req_pos, D.req_game, D.req_stage, D.req_mark, D.req_count, D.logits, D.values, D.cache_tag,
                     D.cache_exps, D.cache_tot, D.cache_val, D.req_out, D.records,
                     D.done, D.done_count, grp.d_done_snapshot, grp.d_status, grp.d_timed_evals, grp.d_features, grp.d_offsets, grp.d_stage};
     for (void *p : ptrs)
@@ -467,14 +468,11 @@ extern "C" int az_pool_create(az_context *ctx, const az_pool_config *cfg, az_poo
         }
         // the level budget trims the tail of a tick over thousands of games; a handful of trees has no tail to trim, and a
         // suspended descent would cost it a whole (empty) net launch
-        // Capped pools (thousands of games, the net launch is full anyway) bound a game's share of a tick in CLOCKS -- 105 k, a
-        // budget a game spends on whatever it has to do (a game that resumes a suspended descent has no evaluation to consume
-        // and gets further) -- with a wide level bound behind it; +0.6 % over 48 levels in three A/B sweeps
-        // (profiles/r02_tree_phases.txt).  Pools of a few hundred games keep the level budget alone.
-        const bool capped = D.cap < D.G;
-        D.levels_per_tick = getenv("AZ_LEVELS_PER_TICK") ? atoi(getenv("AZ_LEVELS_PER_TICK")) : (cfg->games < 64 ? (1 << 20) : capped ? 200 : 48);
+        // No default budget is in clock cycles: how far a game gets would then depend on timing, and the same seed would
+        // not replay the same games (AZ_TICK_CYCLES sets one for experiments).
+        D.levels_per_tick = getenv("AZ_LEVELS_PER_TICK") ? atoi(getenv("AZ_LEVELS_PER_TICK")) : (cfg->games < 64 ? (1 << 20) : 48);
         D.seed = cfg->seed;
-        D.tick_cycles = getenv("AZ_TICK_CYCLES") ? atoi(getenv("AZ_TICK_CYCLES")) : (capped && !getenv("AZ_LEVELS_PER_TICK") ? 105000 : 0);
+        D.tick_cycles = getenv("AZ_TICK_CYCLES") ? atoi(getenv("AZ_TICK_CYCLES")) : 0;
         D.prefetch = getenv("AZ_TREE_PREFETCH") ? atoi(getenv("AZ_TREE_PREFETCH")) : 8;
         D.force_slow = getenv("AZ_TREE_FORCE_SLOW") ? atoi(getenv("AZ_TREE_FORCE_SLOW")) : 0;
         D.one_random_move = (cfg->auto_play && cfg->one_random_move) ? 1 : 0;
@@ -486,6 +484,8 @@ extern "C" int az_pool_create(az_context *ctx, const az_pool_config *cfg, az_poo
         rc |= dev_alloc(&D.gstack, G * D.C, false);
         rc |= dev_alloc(&D.req_pos, G);
         rc |= dev_alloc(&D.req_game, G);
+        rc |= dev_alloc(&D.req_stage, G);
+        rc |= dev_alloc(&D.req_mark, G);          // zero: no tick 0 is ever launched
         rc |= dev_alloc(&D.req_count, 8);
         rc |= dev_alloc(&D.logits, G * AZ_LOGITS);
         rc |= dev_alloc(&D.values, G);

@@ -131,6 +131,9 @@ struct PoolDev {
     uint32_t *gstack;        // [G][C]
     az_position *req_pos;    // [G]
     int32_t *req_game;       // [G]
+    az_position *req_stage;  // [G] a game's request of this tick, by game index (internal net, no cache)
+    uint64_t *req_mark;      // [G] tick_id << 1 | 0 (request deferred last tick) / 1 (new request); k_order_requests lays
+                             // the marked requests of this tick out in req_pos in an order that does not depend on timing
     int32_t *req_count;      // [3 slots][2]: {requests, games that still have work but made no request} of a tick.  Ticks
                              // rotate through the slots (tick_slot); a tick reads its predecessor's request count (of which
                              // the first `cap` were evaluated) and zeroes its successor's slot, so the host never memsets.

@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference's CPU pipeline
+    python bench.py --dump-outputs DIR ...                          # our arm, plus the timed path's outputs as DIR/*.npy
 
 Workload (config.workload): the per-GPU shard of BASELINE configs[3] -- 2048 concurrent self-play
 games x 800 visits/move, random-init model-001 net (bf16 tensor-core mode), Dirichlet noise on,
@@ -338,6 +339,47 @@ def synthetic_roots(ctx, n, seed):
     return arr
 
 
+DUMP_GAMES = 2048                 # roots written by --dump-outputs: 2048 games x 256 move slots x 24 bytes = 12.6 MB
+
+
+def dump_outputs(directory, pool, counters):
+    """--dump-outputs: the state the timed steps leave in the pool, one .npy per array.  For every game: the root position
+    (ply, turn, blockers, x, o), the per-move root statistics in movegen order (packed move, visits, total score, prior;
+    -1 / 0 past the game's move count), the root's visits and value; plus the counters of the timed region.  The game
+    records that selfplay_ticks hands its caller are not dumped: the timed steps keep them on the device, and the root state
+    stands in for them at a fixed size.  Pools of more than DUMP_GAMES games write the same seeded sample of them every run;
+    under torchrun only rank 0 writes.
+
+    The same arguments give the same files: the pool replays its games exactly from the seed (which requests a tick's net
+    launch serves, and how far a game gets in a tick, do not depend on timing), so two builds compare array for array."""
+    import numpy as np
+    from ataxxzero_b200 import rules
+    from ataxxzero_b200._native import AZ_MAX_MOVES
+    games = pool.games
+    idx = np.arange(games)
+    if games > DUMP_GAMES:
+        idx = np.sort(np.random.default_rng(0).choice(games, DUMP_GAMES, replace=False))
+    n = len(idx)
+    out = {"game_index": idx.astype(np.float64), "root_position": np.zeros((n, 5)),
+           "root_moves": np.full((n, AZ_MAX_MOVES), -1.0, np.float32), "root_edge_visits": np.zeros((n, AZ_MAX_MOVES), np.float32),
+           "root_total_score": np.zeros((n, AZ_MAX_MOVES)), "root_prior": np.zeros((n, AZ_MAX_MOVES)),
+           "root_visits": np.zeros(n), "root_value": np.zeros(n)}
+    for row, g in enumerate(idx):
+        r = pool.root(int(g))
+        p, k = r["position"], len(r["moves"])
+        out["root_position"][row] = (p.ply, p.turn, p.blockers, p.pieces[0], p.pieces[1])    # bitboards < 2^49: exact in float64
+        out["root_moves"][row, :k] = [rules.pack_move(m) for m in r["moves"]]
+        out["root_edge_visits"][row, :k] = r["visits"]
+        out["root_total_score"][row, :k] = r["total_score"]
+        out["root_prior"][row, :k] = r["prior"]
+        out["root_visits"][row], out["root_value"][row] = r["root_visits"], r["value"]
+    names = ("ticks", "steps", "evals", "terminal_steps", "positions", "games_finished", "games_skipped")
+    out["timed_counters"] = np.array([counters[name] for name in names], np.float64)      # in the order of `names`
+    os.makedirs(directory, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(directory, name + ".npy"), arr)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -373,7 +415,7 @@ def run_ours(args):
             dist.all_reduce(t, op=dist.ReduceOp.SUM if op == "sum" else dist.ReduceOp.MAX)
         return float(t.item())
 
-    k, w = max(args.steps, 1), max(args.warmup, 3)
+    k, w = args.steps, max(args.warmup, 3)
     games, visits, ticks = args.games, args.visits, args.ticks_per_step
     ctx = az.Context(device=local_rank, seed=azdist.rank_seed(1000, rank))
     network = model.Network.random_init(seed=0)          # "model-001": the reference's init distributions
@@ -409,6 +451,8 @@ def run_ours(args):
     evals = allreduce(d["evals"])
     steps = allreduce(d["steps"])
     value = positions / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pool, d)
 
     # ---- roofline of the dominant kernel (net), from CUDA events around its launches ----
     pk, pk_kind = peaks()
@@ -431,8 +475,8 @@ def run_ours(args):
                 "peak_kind": "%s bf16_tflops_sustained (kernel timed inside a long step)" % pk_kind,
                 "net_share_of_step": d["net_seconds"] / max(d["net_seconds"] + d["tree_seconds"], 1e-9),
                 "tree_ms_per_tick": d["tree_seconds"] / timed * 1e3, "net_ms_per_tick": d["net_seconds"] / timed * 1e3,
-                "launches_timed": int(2 * timed), "evals_timed": int(timed_evals),
-                "timing": "CUDA events around every k_tree_tick and k_net_pair launch of %d ticks (contiguous 256-tick windows, one per 1024 "
+                "launches_timed": int(3 * timed), "evals_timed": int(timed_evals),
+                "timing": "CUDA events around every k_tree_tick (with the k_order_requests behind it) and k_net_pair launch of %d ticks (contiguous 256-tick windows, one per 1024 "
                           "ticks of the timed region), summed; the evaluations of exactly those net launches are counted on the device; "
                           "ticks outside the windows carry no events (an event between two kernels costs ~3 us)" % timed}
     # tree kernel: HBM roofline on SURVEY 8(d)'s algorithmic bytes of the reference algorithm (13 KB per MCTS step: every
@@ -658,10 +702,17 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def positive_int(text):
+    value = int(text)
+    if value < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %d" % value)
+    return value
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=4)
+    ap.add_argument("--steps", type=positive_int, default=4, help="timed steps of TICKS_PER_STEP ticks each")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "counted"])
     ap.add_argument("--games", type=int, default=GAMES_PER_GPU)
@@ -671,6 +722,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-single-tree", action="store_true")
     ap.add_argument("--single-tree-visits", type=int, default=100000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed (see dump_outputs) to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "counted":         # helper of the cpu_baseline leg (see reference_sample)
         import ataxxzero_b200 as az

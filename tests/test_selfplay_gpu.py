@@ -63,6 +63,29 @@ def test_selfplay_noise_changes_games_and_seed_reproduces(tmp_path, ctx):
     assert a != c
 
 
+def test_capped_pool_replays_bit_for_bit(ctx, monkeypatch):
+    """A capped pool -- the net serves only the first `cap` requests of a tick, the rest wait a tick -- replays exactly: which
+    requests are served and how far each game gets in a tick follow from the seed, not from when the tree kernel's warps
+    finish.  Same seed, same ticks: every root and every counter is the same, bit for bit."""
+    from ataxxzero_b200 import model, net, search
+    net.load_weights(ctx, model.Network.random_init(seed=0))
+    monkeypatch.setenv("AZ_REQ_CAP", "160")         # read when the pool is created: far fewer than the 512 games request
+
+    def run():
+        with search.Pool(ctx, 512, 64, eval_mode=search.EVAL_BF16, noise=True, auto_play=True, seed=5) as pool:
+            st = pool.selfplay_ticks(300)
+            return st, [pool.root(g) for g in range(512)]
+    (sa, ra), (sb, rb) = run(), run()
+    assert sa["positions"] > 0 and sa["evals"] <= 160 * 300 + 512       # the cap bound: requests really were deferred
+    for key in ("ticks", "steps", "evals", "terminal_steps", "positions", "games_finished", "max_depth", "levels"):
+        assert sa[key] == sb[key], key
+    for x, y in zip(ra, rb):
+        assert x["position"].key() == y["position"].key() and x["position"].ply == y["position"].ply
+        assert x["moves"] == y["moves"] and x["visits"] == y["visits"] and x["root_visits"] == y["root_visits"]
+        assert [float(v).hex() for v in x["total_score"]] == [float(v).hex() for v in y["total_score"]]
+        assert [float(v).hex() for v in x["prior"]] == [float(v).hex() for v in y["prior"]]
+
+
 def test_visit_targets_respected(tmp_path, ctx, oracle):
     """Each recorded distribution is n/N with N >= visits at the moment the move was chosen."""
     from ataxxzero_b200 import model, net, search

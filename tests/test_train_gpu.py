@@ -183,6 +183,7 @@ def test_resident_games_step_equals_host_minibatch_step(ctx):
     network = model.Network.random_init(seed=3, blocks=1)
     a, b = trainer.Trainer(ctx, network, max_batch=64), trainer.Trainer(ctx, network, max_batch=64)
     a.set_games(packed)
+    w0 = network.conv[1]
     rng = np.random.default_rng(2)
     for step in range(3):
         offsets, meta = train_data.draw_arrays(packed, 64, rng)
@@ -199,7 +200,14 @@ def test_resident_games_step_equals_host_minibatch_step(ctx):
         # step (DESIGN 3g: like the reference's TensorFlow step it is not bit-reproducible); after that the two trainers'
         # weights drift apart by that rounding, amplified by the momentum updates (observed: 1.2e-5 relative at step 2)
         assert np.allclose(la, lb, rtol=1e-5 if step == 0 else 5e-4, atol=1e-6), (step, la, lb)
-    assert np.allclose(a.debug_read("conv", 1), b.debug_read("conv", 1), rtol=2e-3, atol=1e-5)
+        wa, wb = a.debug_read("conv", 1), b.debug_read("conv", 1)
+        if step < 2:
+            assert np.allclose(wa, wb, rtol=2e-3, atol=1e-5), step
+    # by the third step one rounding flip in those sums can move a few hundred of this layer's weights by up to 8e-5, and it
+    # does so between two trainers on the SAME path as often (measured on a B200 at 1000 W: in 2 of 6 runs one of three
+    # trainers flipped, by 0.6 - 0.75 % of the layer's update): past that point the two paths are held to taking the same
+    # update, not to the same rounding.  The 2 % bound is 2.7x the largest flip of those six runs, no more data than that.
+    assert np.linalg.norm(wa - wb) < 2e-2 * np.linalg.norm(wb - w0), (np.linalg.norm(wa - wb), np.linalg.norm(wb - w0))
     bad = offsets.copy()
     bad[5] = packed.words.size                                 # outside the table
     with pytest.raises(AzError):

@@ -283,6 +283,14 @@ extern "C" int az_net_forward_dev(az_context *ctx, const void *d_features, int n
     return net_forward_dev(ctx, d_features, AZ_IN_F32, n, mode, d_logits, d_values);
 }
 
+// Test hook (not part of the public header): a forward pass over min(*d_count, n) boards, the count read from device memory
+// when the kernel starts -- the way the self-play pool launches the net behind the tree kernel.
+extern "C" int az_net_forward_counted_dev(az_context *ctx, const void *d_features, int n, const int *d_count, int mode, void *d_logits, void *d_values)
+{
+    AZ_REQUIRE(d_count, AZ_ERR_ARG, "az_net_forward_counted_dev: no count");
+    return net_forward_dev(ctx, d_features, AZ_IN_F32, n, mode, d_logits, d_values, d_count);
+}
+
 extern "C" int az_net_forward_pos_dev(az_context *ctx, const void *d_pos, int n, int mode, void *d_logits, void *d_values)
 {
     return net_forward_dev(ctx, d_pos, AZ_IN_POS, n, mode, d_logits, d_values);

@@ -36,6 +36,9 @@ struct AzNet {
     uint8_t *pair_stream = nullptr;    // CTA-pair kernel (az_net_pair.cu): every stage split into the two CTAs' output-channel halves
     uint8_t *pair_stream16 = nullptr;
     int tc_pair = 0;                   // 1: plain forward passes run on CTA pairs (tcgen05 cta_group::2)
+    int pair_tiles = 0;                // tiles per CTA of the pair kernel: 1, 2, or 0 = 2 for batches of a full round, else 1
+    long long *pair_prof = nullptr;    // issuer wait records of k_net_pair (az_net_pair_profile; profiling only)
+    int pair_prof_max = 0;
     int tc_tiles = 2;                  // kernel variant: tiles (of 2 boards) per CTA
     int tc_cluster = 1;                // CTAs per cluster sharing one multicast weight stream
     __nv_bfloat16 *tc_w = nullptr;     // [2*blocks][18 chunks][8 kgroups][128 cout][8 cin]

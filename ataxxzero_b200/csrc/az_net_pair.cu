@@ -45,25 +45,35 @@ constexpr int HEAD_HALF = HEAD_N / 2;
 constexpr int WHEAD_HALF_BYTES = KG * HEAD_HALF * ROW_BYTES;   // 4 KiB
 constexpr int HEAD_LBO = HEAD_HALF * ROW_BYTES;
 
-constexpr int STAGES = 8;                // 64 KiB of weight stages in flight per CTA
 constexpr int ACT_ROWS = MARGIN + TILE_M + MARGIN;
 constexpr int ACT_LBO = ACT_ROWS * ROW_BYTES;
-constexpr int ACT_BYTES = KG * ACT_LBO;
-constexpr int OFF_ACT = 0;
-constexpr int OFF_IN = OFF_ACT;          // input planes are staged in k-group 0 of the activation buffer
-constexpr int OFF_RING = OFF_ACT + ACT_BYTES;
-constexpr int OFF_SHIFT = OFF_RING + STAGES * STAGE_BYTES;     // float[2][F]
-constexpr int OFF_VPART = OFF_SHIFT + 2 * F * 4;
-constexpr int OFF_BAR = OFF_VPART + 64;
-constexpr int B_FULL = 0, B_EMPTY = STAGES, B_ACC = 2 * STAGES, B_ACT = 2 * STAGES + 1, B_IN = 2 * STAGES + 1 + SPLIT;
-constexpr int NUM_BARS = B_IN + 1;
-constexpr int OFF_TMEM = OFF_BAR + NUM_BARS * 8;
-constexpr int SMEM_BYTES = OFF_TMEM + 16;
-constexpr int NUM_WARPS = 6;
-constexpr int NUM_THREADS = NUM_WARPS * 32;
-constexpr int UNIT_BOARDS = 2;
-constexpr uint32_t TMEM_COLS = 256, TM_ACC = 0, TM_RES = 128;
-static_assert(SMEM_BYTES * 2 + 2048 <= 228 * 1024, "two CTAs per SM");
+constexpr int ACT_BYTES = KG * ACT_LBO;  // one tile's activations; its input planes are staged in k-group 0
+constexpr uint32_t TM_ACC = 0, TM_RES = 128, TM_TILE = 256;    // per tile: accumulator + residual columns
+constexpr int ACC = 0, ACT = 1, IN = 1 + SPLIT, TILE_BARS = 2 + SPLIT;   // per-tile barriers: accumulator, activation parts, input
+
+// TILES = 1: two CTAs (two unrelated pairs) per SM, one 128-row tile each.  TILES = 2: one CTA per SM with two tiles that
+// consume every weight stage one after the other, so that each tile's epilogue runs behind the other tile's MMAs (see the issuer).
+template <int TILES>
+struct PairCfg {
+    static constexpr int STAGES = 8 * TILES;                    // TILES = 2: a stage stays live for 9 chunks of tile 0
+    static constexpr int OFF_ACT = 0;                           // one activation buffer per tile
+    static constexpr int OFF_RING = OFF_ACT + TILES * ACT_BYTES;
+    static constexpr int OFF_SHIFT = OFF_RING + STAGES * STAGE_BYTES;   // float[TILES][2][F]
+    static constexpr int OFF_VPART = OFF_SHIFT + TILES * 2 * F * 4;     // float[TILES][16]
+    static constexpr int OFF_BAR = OFF_VPART + TILES * 64;
+    static constexpr int B_FULL = 0, B_EMPTY = STAGES, B_TILE = 2 * STAGES;
+    static constexpr int NUM_BARS = B_TILE + TILES * TILE_BARS;
+    static constexpr int OFF_TMEM = OFF_BAR + NUM_BARS * 8;
+    static constexpr int SMEM_BYTES = OFF_TMEM + 16;
+    static constexpr int NUM_WARPS = 2 + 4 * TILES;             // producer, issuer / relay, 4 epilogue warps per tile
+    static constexpr int NUM_THREADS = NUM_WARPS * 32;
+    static constexpr int UNIT_BOARDS = 2 * TILES;
+    static constexpr int CTAS_PER_SM = TILES == 1 ? 2 : 1;
+    static constexpr uint32_t TMEM_COLS = TM_TILE * TILES;
+};
+static_assert(PairCfg<1>::SMEM_BYTES * 2 + 2048 <= 228 * 1024, "two CTAs per SM");
+static_assert(PairCfg<2>::SMEM_BYTES + 1024 <= 228 * 1024, "one two-tile CTA per SM");
+static_assert(PairCfg<2>::STAGES - 9 >= 4, "the ring must prefetch while a part's nine stages wait for the second tile");
 
 // instruction descriptor: D=f32, A/B bf16 (bits 7, 10; cleared for IEEE half), K-major both, N >> 3 at bit 17, M >> 4 at bit 24.
 // M is the PAIR's: 256.
@@ -176,7 +186,12 @@ __device__ __forceinline__ uint32_t pack_op(float lo, float hi, int f16)
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t *>(&v);
 }
-__device__ __forceinline__ void group_sync() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
+// the 128 epilogue threads of one tile (immediate barrier ids: a register operand would reserve all 16 barriers)
+__device__ __forceinline__ void group_sync(int tile)
+{
+    if (tile == 0) asm volatile("bar.sync 1, 128;" ::: "memory");
+    else asm volatile("bar.sync 2, 128;" ::: "memory");
+}
 
 struct PairParams {
     const void *input;                 // float[n][196] or az_position[n]
@@ -189,7 +204,14 @@ struct PairParams {
     float *logits, *values;
     int f16;
     int relay_mode;                    // AZ_PAIR_RELAY: 0 one thread / release arrives, 1 one thread / relaxed arrives, 2 one lane per event stream
+    long long *prof;                   // issuer wait records (k_net_pair<..., true> only, see az_net_pair_profile)
+    int prof_max;                      // records per CTA
 };
+
+// Issuer wait records of the profiling instantiation: per CTA a header {smid, clock at start, clock at end, records} and records
+// {kind + 256 * layer, t0, t1} in clock64() cycles.  Layer 0 is the input conv, 1..nl the tower, nl + 1 the heads.
+enum : int { PROF_GAP = 0, PROF_ACT0 = 1, PROF_ACT1 = 2, PROF_FULL = 3, PROF_IN = 4, PROF_UNIT_GAP = 5 };
+constexpr int PROF_HDR = 4;
 
 __device__ __forceinline__ bool row_is_real(int r, int &board_in_tile, int &cell)
 {
@@ -200,15 +222,20 @@ __device__ __forceinline__ bool row_is_real(int r, int &board_in_tile, int &cell
     return w >= 8 && y != 7;
 }
 
-template <int IN_KIND>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_net_pair(const PairParams P)
+template <int TILES, int IN_KIND, bool PROF>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PairCfg<TILES>::NUM_THREADS, PairCfg<TILES>::CTAS_PER_SM) k_net_pair(const PairParams P)
 {
+    using C = PairCfg<TILES>;
+    constexpr int STAGES = C::STAGES, NUM_THREADS = C::NUM_THREADS, UNIT_BOARDS = C::UNIT_BOARDS;
+    constexpr int OFF_ACT = C::OFF_ACT, OFF_RING = C::OFF_RING, B_FULL = C::B_FULL, B_EMPTY = C::B_EMPTY;
+    static_assert(!PROF || TILES == 1, "wait records are taken for the one-tile schedule");
     const uint32_t crank = cluster_ctarank();
     const bool leader = crank == 0;
     extern __shared__ __align__(1024) uint8_t smem[];
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    auto bar = [&](int i) { return sbase + OFF_BAR + 8 * i; };
+    auto bar = [&](int i) { return sbase + C::OFF_BAR + 8 * i; };
+    auto tbar = [&](int tile, int i) { return bar(C::B_TILE + tile * TILE_BARS + i); };     // per-tile barrier i (ACC, ACT + part, IN)
 
     const int n_boards = P.n_ptr ? min(*P.n_ptr, P.n) : P.n;
     const int num_units = ((n_boards + UNIT_BOARDS - 1) / UNIT_BOARDS + 1) / 2 * 2;      // both CTAs of a pair run the same passes
@@ -216,23 +243,25 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
     const uint32_t idesc_128 = make_idesc(128, P.f16 != 0), idesc_head = make_idesc(HEAD_N, P.f16 != 0);
 
     // ---- one-time setup ----
-    for (int i = threadIdx.x; i < ACT_BYTES / 16; i += NUM_THREADS) reinterpret_cast<uint4 *>(smem + OFF_ACT)[i] = make_uint4(0, 0, 0, 0);
+    for (int i = threadIdx.x; i < TILES * ACT_BYTES / 16; i += NUM_THREADS) reinterpret_cast<uint4 *>(smem + OFF_ACT)[i] = make_uint4(0, 0, 0, 0);
     if (threadIdx.x == 0) {
         // barriers the issuing thread waits on count the peer's relay as one more arrival (leader only)
         const uint32_t extra = leader ? 1u : 0u;
         for (int s = 0; s < STAGES; ++s) { mbar_init(bar(B_FULL + s), 1 + extra); mbar_init(bar(B_EMPTY + s), 1); }
-        mbar_init(bar(B_ACC), 1);
-        for (int p = 0; p < SPLIT; ++p) mbar_init(bar(B_ACT + p), 128 + extra);
-        mbar_init(bar(B_IN), 128 + extra);
+        for (int t = 0; t < TILES; ++t) {
+            mbar_init(tbar(t, ACC), 1);
+            for (int p = 0; p < SPLIT; ++p) mbar_init(tbar(t, ACT + p), 128 + extra);
+            mbar_init(tbar(t, IN), 128 + extra);
+        }
         fence_barrier_init();
     }
-    if (warp == 1) tmem_alloc(sbase + OFF_TMEM, TMEM_COLS);
+    if (warp == 1) tmem_alloc(sbase + C::OFF_TMEM, C::TMEM_COLS);
     fence_proxy_async();
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();                  // the peer's barriers and zero-filled activations exist before anything refers to them
     tc_fence_after();
-    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(smem + OFF_TMEM);
+    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(smem + C::OFF_TMEM);
 
     // chunk sequence of one unit (identical in producer, issuer and relay): input conv (2 stages), nl x 18 tower chunks, heads
     if (warp == 0) {
@@ -263,7 +292,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
         const int pushes_per_unit = (5 + WIN_KSTEPS_PER_STAGE - 1) / WIN_KSTEPS_PER_STAGE + nl * CHUNKS + 1;
         if (P.relay_mode == 2) {
             // every barrier is its own event stream with self-consistent phases: one lane per stream, so that a slow hop on one
-            // of them never delays the others (8 weight stages, the two activation parts, the staged input)
+            // of them never delays the others (the weight stages; per tile the two activation parts and the staged input)
+            static_assert(STAGES + TILES * (SPLIT + 1) <= 32, "one relay lane per event stream");
             const bool relaxed = true;
             if (lane < STAGES) {
                 const uint32_t total = (uint32_t)my_units * (uint32_t)pushes_per_unit;
@@ -271,20 +301,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
                     mbar_wait(bar(B_FULL + lane), (it / STAGES) & 1);
                     mbar_arrive_remote(bar(B_FULL + lane), 0, relaxed);
                 }
-            } else if (lane < STAGES + SPLIT) {
-                const int part = lane - STAGES;
-                const uint32_t total = (uint32_t)my_units * (uint32_t)(nl + 1);
-                for (uint32_t k = 0; k < total; ++k) {
-                    mbar_wait(bar(B_ACT + part), k & 1);
-                    mbar_arrive_remote(bar(B_ACT + part), 0, relaxed);
-                }
-            } else if (lane == STAGES + SPLIT) {
-                for (uint32_t k = 0; k < (uint32_t)my_units; ++k) {
-                    mbar_wait(bar(B_IN), k & 1);
-                    mbar_arrive_remote(bar(B_IN), 0, relaxed);
+            } else if (lane < STAGES + TILES * (SPLIT + 1)) {
+                const int tile = (lane - STAGES) / (SPLIT + 1), k = (lane - STAGES) % (SPLIT + 1);     // k < SPLIT: part k, else input
+                const uint32_t b = tbar(tile, k < SPLIT ? ACT + k : IN);
+                const uint32_t total = (uint32_t)my_units * (uint32_t)(k < SPLIT ? nl + 1 : 1);
+                for (uint32_t e = 0; e < total; ++e) {
+                    mbar_wait(b, e & 1);
+                    mbar_arrive_remote(b, 0, relaxed);
                 }
             }
-        } else if (elect_one()) {
+        } else if (TILES == 1 && elect_one()) {
             const bool relaxed = P.relay_mode == 1;
             uint32_t it = 0, in_phase = 0, act_phase = 0;
             auto relay_stage = [&]() {
@@ -294,21 +320,21 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
                 ++it;
             };
             for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
-                mbar_wait(bar(B_IN), in_phase);
+                mbar_wait(tbar(0, IN), in_phase);
                 in_phase ^= 1;
-                mbar_arrive_remote(bar(B_IN), 0, relaxed);
+                mbar_arrive_remote(tbar(0, IN), 0, relaxed);
                 for (int j0 = 0; j0 < 5; j0 += WIN_KSTEPS_PER_STAGE) relay_stage();
                 for (int l = 0; l < nl; ++l) {
                     for (int part = 0; part < SPLIT; ++part) {
-                        mbar_wait(bar(B_ACT + part), act_phase);
-                        mbar_arrive_remote(bar(B_ACT + part), 0, relaxed);
+                        mbar_wait(tbar(0, ACT + part), act_phase);
+                        mbar_arrive_remote(tbar(0, ACT + part), 0, relaxed);
                         for (int tap = 0; tap < 9; ++tap) relay_stage();
                     }
                     act_phase ^= 1;
                 }
                 for (int p = 0; p < SPLIT; ++p) {
-                    mbar_wait(bar(B_ACT + p), act_phase);
-                    mbar_arrive_remote(bar(B_ACT + p), 0, relaxed);
+                    mbar_wait(tbar(0, ACT + p), act_phase);
+                    mbar_arrive_remote(tbar(0, ACT + p), 0, relaxed);
                 }
                 act_phase ^= 1;
                 relay_stage();
@@ -316,93 +342,153 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
         }
     } else if (warp == 1) {
         // =============================== MMA issuer (leader): one M=256 MMA per step for the pair ===============================
+        // TILES = 2: the tiles take every weight stage one after the other -- per layer t0.part0, t1.part0, t0.part1, t1.part1 --
+        // so tile 1 runs half a layer behind tile 0.  Tile 0's epilogue of layer l then runs behind t1.part1(l), and t0.part0(l+1)
+        // needs only its first half; tile 1's epilogue runs behind t0.part0(l+1) in the same way.  A stage is freed after the last
+        // tile's MMAs on it (9 chunks after the first tile's), hence the 16-stage ring.  Per tile, the operands, the chunk order
+        // and the accumulation are those of TILES = 1: the results are identical bit for bit.
         if (elect_one()) {
             uint32_t it = 0, in_phase = 0, act_phase = 0;
+            // PROF: the issuer also waits for each accumulator commit before the wait that follows it anyway, to time the
+            // stretch in which this pair has no MMA queued ("gap": accumulator done -> next layer's first input part ready)
+            long long *rec = PROF ? P.prof + (size_t)blockIdx.x * (PROF_HDR + 3 * P.prof_max) : nullptr;
+            int nrec = 0;
+            uint32_t acc_ph = 0;
+            long long t_acc = 0, full_sum = 0;
+            auto note = [&](int kind, int layer, long long t0, long long t1) {
+                if (PROF && nrec < P.prof_max) {
+                    rec[PROF_HDR + 3 * nrec] = kind + 256 * layer; rec[PROF_HDR + 3 * nrec + 1] = t0; rec[PROF_HDR + 3 * nrec + 2] = t1;
+                    ++nrec;
+                }
+            };
+            auto acc_done = [&]() {
+                if (PROF) { mbar_wait(tbar(0, ACC), acc_ph); acc_ph ^= 1; t_acc = clock64(); }
+            };
+            auto full_wait = [&](int s, uint32_t parity) {
+                const long long t0 = PROF ? clock64() : 0;
+                mbar_wait(bar(B_FULL + s), parity);
+                if (PROF) full_sum += clock64() - t0;
+            };
+            if (PROF) { uint32_t smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); rec[0] = smid; rec[1] = clock64(); t_acc = rec[1]; }
             auto acquire = [&]() {
                 const int s = it % STAGES;
-                mbar_wait(bar(B_FULL + s), (it / STAGES) & 1);
+                full_wait(s, (it / STAGES) & 1);
                 tc_fence_after();
                 return sbase + OFF_RING + s * STAGE_BYTES;
             };
             auto release = [&]() { umma2_commit(bar(B_EMPTY + it % STAGES)); ++it; };
+            const uint32_t a_hi = (uint32_t)(make_desc(0, ACT_LBO) >> 32), b_hi = (uint32_t)(make_desc(0, W_LBO) >> 32);
+            const uint32_t a_lo0 = (uint32_t)make_desc(sbase + OFF_ACT + MARGIN * ROW_BYTES, ACT_LBO);
+            const uint32_t b_lo0 = (uint32_t)make_desc(sbase + OFF_RING, W_LBO);
+            constexpr uint32_t A_KSTEP = (2 * ACT_LBO) >> 4, B_KSTEP = (2 * W_LBO) >> 4, A_PART = (PART_KG * ACT_LBO) >> 4, A_TILE = ACT_BYTES >> 4;
             for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
                 // ---- input conv: 9 taps x 8 (4 real) channels, two taps per K=16 step ----
-                mbar_wait(bar(B_IN), in_phase);
-                in_phase ^= 1;
-                tc_fence_after();
                 for (int j0 = 0; j0 < 5; j0 += WIN_KSTEPS_PER_STAGE) {
                     const uint32_t b_rows = acquire();
                     const int j1 = min(j0 + WIN_KSTEPS_PER_STAGE, 5);
-                    const uint32_t in_rows = sbase + OFF_IN + MARGIN * ROW_BYTES;
-                    for (int j = j0; j < j1; ++j) {
-                        const int tap0 = 2 * j, tap1 = 2 * j + 1;
-                        const uint32_t a0 = in_rows + ((tap0 / 3 - 1) * 8 + (tap0 % 3 - 1)) * ROW_BYTES;
-                        const uint32_t a1 = tap1 < 9 ? in_rows + ((tap1 / 3 - 1) * 8 + (tap1 % 3 - 1)) * ROW_BYTES : a0 + ROW_BYTES;   // 10th tap: zero weights
-                        umma2(tmem_base + TM_ACC, make_desc(a0, a1 - a0), make_desc(b_rows + (j - j0) * 2 * W_LBO, W_LBO), idesc_128, j > 0);
+#pragma unroll
+                    for (int t = 0; t < TILES; ++t) {
+                        if (j0 == 0) {
+                            const long long t0 = PROF ? clock64() : 0;
+                            mbar_wait(tbar(t, IN), in_phase);
+                            if (PROF) { const long long t1 = clock64(); note(PROF_IN, 0, t0, t1); note(PROF_UNIT_GAP, 0, t_acc, t1); }
+                            tc_fence_after();
+                        }
+                        const uint32_t in_rows = sbase + OFF_ACT + t * ACT_BYTES + MARGIN * ROW_BYTES;
+                        for (int j = j0; j < j1; ++j) {
+                            const int tap0 = 2 * j, tap1 = 2 * j + 1;
+                            const uint32_t a0 = in_rows + ((tap0 / 3 - 1) * 8 + (tap0 % 3 - 1)) * ROW_BYTES;
+                            const uint32_t a1 = tap1 < 9 ? in_rows + ((tap1 / 3 - 1) * 8 + (tap1 % 3 - 1)) * ROW_BYTES : a0 + ROW_BYTES;   // 10th tap: zero weights
+                            umma2(tmem_base + t * TM_TILE + TM_ACC, make_desc(a0, a1 - a0), make_desc(b_rows + (j - j0) * 2 * W_LBO, W_LBO), idesc_128, j > 0);
+                        }
+                        if (j1 == 5) umma2_commit(tbar(t, ACC));
                     }
-                    if (j1 == 5) umma2_commit(bar(B_ACC));
                     release();
                 }
+                in_phase ^= 1;
                 // ---- tower ----
-                const uint32_t a_hi = (uint32_t)(make_desc(0, ACT_LBO) >> 32), b_hi = (uint32_t)(make_desc(0, W_LBO) >> 32);
-                const uint32_t a_lo0 = (uint32_t)make_desc(sbase + OFF_ACT + MARGIN * ROW_BYTES, ACT_LBO);
-                const uint32_t b_lo0 = (uint32_t)make_desc(sbase + OFF_RING, W_LBO);
-                constexpr uint32_t A_KSTEP = (2 * ACT_LBO) >> 4, B_KSTEP = (2 * W_LBO) >> 4, A_PART = (PART_KG * ACT_LBO) >> 4;
                 for (int l = 0; l < nl; ++l) {
                     const uint32_t onto_res = (uint32_t)(l & 1);        // second conv of a block: on top of the residual columns
-                    const uint32_t d_col = tmem_base + (onto_res ? TM_RES : TM_ACC);
+                    if (PROF) { note(PROF_FULL, l, 0, full_sum); full_sum = 0; acc_done(); }
 #pragma unroll 1
                     for (int part = 0; part < SPLIT; ++part) {
-                        mbar_wait(bar(B_ACT + part), act_phase);
-                        tc_fence_after();
 #pragma unroll
-                        for (int tap = 0; tap < 9; ++tap) {
-                            const int s = it % STAGES;
-                            mbar_wait(bar(B_FULL + s), (it / STAGES) & 1);
+                        for (int t = 0; t < TILES; ++t) {
+                            const uint32_t d_col = tmem_base + t * TM_TILE + (onto_res ? TM_RES : TM_ACC);
+                            {
+                                const long long t0 = PROF ? clock64() : 0;
+                                mbar_wait(tbar(t, ACT + part), act_phase);
+                                if (PROF) {
+                                    const long long t1 = clock64();
+                                    note(part ? PROF_ACT1 : PROF_ACT0, l + 1, t0, t1);
+                                    if (part == 0) note(PROF_GAP, l + 1, t_acc, t1);
+                                }
+                            }
                             tc_fence_after();
-                            const uint32_t b_lo = b_lo0 + s * (STAGE_BYTES >> 4);
-                            const uint32_t a_lo = a_lo0 + part * A_PART + (uint32_t)((tap / 3 - 1) * 8 + (tap % 3 - 1));
 #pragma unroll
-                            for (int j = 0; j < PART_MMAS; ++j)
-                                umma2_lo(d_col, a_lo + j * A_KSTEP, a_hi, b_lo + j * B_KSTEP, b_hi, idesc_128, onto_res | (uint32_t)((part | tap | j) != 0));
-                            if (part == SPLIT - 1 && tap == 8) umma2_commit(bar(B_ACC));
-                            umma2_commit(bar(B_EMPTY + s));
-                            ++it;
+                            for (int tap = 0; tap < 9; ++tap) {
+                                const int s = (it + tap) % STAGES;
+                                if (t == 0) {           // the later tiles find the stage landed
+                                    full_wait(s, ((it + tap) / STAGES) & 1);
+                                    tc_fence_after();
+                                }
+                                const uint32_t b_lo = b_lo0 + s * (STAGE_BYTES >> 4);
+                                const uint32_t a_lo = a_lo0 + t * A_TILE + part * A_PART + (uint32_t)((tap / 3 - 1) * 8 + (tap % 3 - 1));
+#pragma unroll
+                                for (int j = 0; j < PART_MMAS; ++j)
+                                    umma2_lo(d_col, a_lo + j * A_KSTEP, a_hi, b_lo + j * B_KSTEP, b_hi, idesc_128, onto_res | (uint32_t)((part | tap | j) != 0));
+                                if (part == SPLIT - 1 && tap == 8) umma2_commit(tbar(t, ACC));
+                                if (t == TILES - 1) umma2_commit(bar(B_EMPTY + s));
+                            }
                         }
+                        it += 9;
                     }
                     act_phase ^= 1;
                 }
                 // ---- heads: [256 rows x 128 ch] x [128 ch x 32] ----
-                for (int p = 0; p < SPLIT; ++p) mbar_wait(bar(B_ACT + p), act_phase);
-                act_phase ^= 1;
-                tc_fence_after();
+                if (PROF) { note(PROF_FULL, nl, 0, full_sum); full_sum = 0; acc_done(); }
                 {
-                    const uint32_t b_rows = acquire();
-                    const uint32_t a_rows = sbase + OFF_ACT + MARGIN * ROW_BYTES;
+                    uint32_t b_rows = 0;
 #pragma unroll
-                    for (int j = 0; j < 8; ++j)
-                        umma2(tmem_base + TM_ACC, make_desc(a_rows + 2 * j * ACT_LBO, ACT_LBO), make_desc(b_rows + 2 * j * HEAD_LBO, HEAD_LBO), idesc_head, j > 0);
-                    umma2_commit(bar(B_ACC));
+                    for (int t = 0; t < TILES; ++t) {
+                        {
+                            const long long t0 = PROF ? clock64() : 0;
+                            for (int p = 0; p < SPLIT; ++p) mbar_wait(tbar(t, ACT + p), act_phase);
+                            if (PROF) { const long long t1 = clock64(); note(PROF_ACT0, nl + 1, t0, t1); note(PROF_GAP, nl + 1, t_acc, t1); }
+                        }
+                        tc_fence_after();
+                        if (t == 0) b_rows = acquire();
+                        const uint32_t a_rows = sbase + OFF_ACT + t * ACT_BYTES + MARGIN * ROW_BYTES;
+#pragma unroll
+                        for (int j = 0; j < 8; ++j)
+                            umma2(tmem_base + t * TM_TILE + TM_ACC, make_desc(a_rows + 2 * j * ACT_LBO, ACT_LBO), make_desc(b_rows + 2 * j * HEAD_LBO, HEAD_LBO),
+                                  idesc_head, j > 0);
+                        umma2_commit(tbar(t, ACC));
+                    }
                     release();
                 }
+                act_phase ^= 1;
+                if (PROF) { note(PROF_FULL, nl + 1, 0, full_sum); full_sum = 0; acc_done(); }
             }
+            if (PROF) { rec[2] = clock64(); rec[3] = nrec; }
         }
     } else {
-        // =============================== epilogue warps (both CTAs, each on its own 128 TMEM lanes) ===============================
-        const int quad = warp & 3;
+        // =============================== epilogue warps (both CTAs, each on its own 128 TMEM lanes of its tile) ===============================
+        const int tile = TILES == 1 ? 0 : (warp - 2) >> 2;
+        const int quad = warp & 3;               // a warp reaches TMEM lanes 32 * (warp % 4) ..
         const int r = quad * 32 + lane;
-        const int gtid = (warp - 2) * 32 + lane;
+        const int gtid = ((warp - 2) & 3) * 32 + lane;
         int bit, cell;
         const bool real = row_is_real(r, bit, cell);
-        float *shift_base = reinterpret_cast<float *>(smem + OFF_SHIFT);
-        float *vpart = reinterpret_cast<float *>(smem + OFF_VPART);
-        const uint32_t lane_addr = tmem_base + ((uint32_t)(quad * 32) << 16);
-        uint8_t *act_row = smem + OFF_ACT + (MARGIN + r) * ROW_BYTES;
+        float *shift_base = reinterpret_cast<float *>(smem + C::OFF_SHIFT) + tile * 2 * F;
+        float *vpart = reinterpret_cast<float *>(smem + C::OFF_VPART) + tile * 16;
+        const uint32_t lane_addr = tmem_base + tile * TM_TILE + ((uint32_t)(quad * 32) << 16);
+        uint8_t *act_row = smem + OFF_ACT + tile * ACT_BYTES + (MARGIN + r) * ROW_BYTES;
         uint32_t acc_phase = 0;
         // "this row's part of the activations is written": locally, and -- in the leader -- that is all; the peer's relay
         // thread forwards the completed phase
         for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
-            const int board = unit * UNIT_BOARDS + bit;
+            const int board = unit * UNIT_BOARDS + tile * 2 + bit;
             const bool live = real && board < n_boards;
             {
                 uint4 v = make_uint4(0, 0, 0, 0);
@@ -419,17 +505,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
                     v.x = pack_op(f[0], f[1], P.f16);
                     v.y = pack_op(f[2], f[3], P.f16);
                 }
-                *reinterpret_cast<uint4 *>(smem + OFF_IN + (MARGIN + r) * ROW_BYTES) = v;
+                *reinterpret_cast<uint4 *>(act_row) = v;         // k-group 0 of the tile's activations
                 fence_proxy_async();
-                mbar_arrive(bar(B_IN));
+                mbar_arrive(tbar(tile, IN));
             }
             for (int l = 0; l < P.layers; ++l) {
                 const bool second = l > 0 && (l & 1) == 0;
                 const bool writes_res = l == 0 || second;
                 float *shift_s = shift_base + (l & 1) * F;
                 shift_s[gtid] = __ldg(P.shift + l * F + gtid);
-                group_sync();
-                mbar_wait(bar(B_ACC), acc_phase);
+                group_sync(tile);
+                mbar_wait(tbar(tile, ACC), acc_phase);
                 acc_phase ^= 1;
                 tc_fence_after();
                 const uint32_t src = lane_addr + (second ? TM_RES : TM_ACC);
@@ -461,17 +547,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
                         // conv: layer 1 reuses the accumulator this epilogue is still reading)
                         fence_proxy_async();
                         tc_fence_before();
-                        mbar_arrive(bar(B_ACT + 0));
+                        mbar_arrive(tbar(tile, ACT + 0));
                     }
                 }
                 if (writes_res) tmem_wait_st();
                 fence_proxy_async();
                 tc_fence_before();
-                if (l == 0) mbar_arrive(bar(B_ACT + 0));
-                mbar_arrive(bar(B_ACT + 1));
+                if (l == 0) mbar_arrive(tbar(tile, ACT + 0));
+                mbar_arrive(tbar(tile, ACT + 1));
             }
             {
-                mbar_wait(bar(B_ACC), acc_phase);
+                mbar_wait(tbar(tile, ACC), acc_phase);
                 acc_phase ^= 1;
                 tc_fence_after();
                 uint32_t a[32];
@@ -488,19 +574,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 2) k_ne
                 for (int s = 16; s; s >>= 1) vterm += __shfl_xor_sync(0xffffffffu, vterm, s);
                 if (lane == 0) vpart[quad] = vterm;
                 tc_fence_before();
-                group_sync();
+                group_sync(tile);
                 if (gtid < 2) {
-                    const int b = unit * UNIT_BOARDS + gtid;
+                    const int b = unit * UNIT_BOARDS + tile * 2 + gtid;
                     if (b < n_boards) P.values[b] = tanhf(vpart[2 * gtid] + vpart[2 * gtid + 1] + __ldg(P.fc_b));
                 }
-                group_sync();
+                group_sync(tile);
             }
         }
     }
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();                  // nobody leaves (or frees tensor memory) while the pair's MMAs may still touch it
-    if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
+    if (warp == 1) tmem_dealloc(tmem_base, C::TMEM_COLS);
 }
 
 // ---- weight tiling for the pair layout ----
@@ -565,8 +651,12 @@ int az_net_pair_alloc(AzNet *net)
     const size_t bytes = az_net_pair_stream_bytes(net);
     AZ_CUDA(cudaMalloc(&net->pair_stream, bytes));
     AZ_CUDA(cudaMalloc(&net->pair_stream16, bytes));
-    AZ_CUDA(cudaFuncSetAttribute(k_net_pair<AZ_IN_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    AZ_CUDA(cudaFuncSetAttribute(k_net_pair<AZ_IN_POS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+#define AZ_PAIR_ATTR(T, K, PROF) AZ_CUDA(cudaFuncSetAttribute(k_net_pair<T, K, PROF>, cudaFuncAttributeMaxDynamicSharedMemorySize, PairCfg<T>::SMEM_BYTES))
+    AZ_PAIR_ATTR(1, AZ_IN_F32, false); AZ_PAIR_ATTR(1, AZ_IN_POS, false); AZ_PAIR_ATTR(1, AZ_IN_F32, true); AZ_PAIR_ATTR(1, AZ_IN_POS, true);
+    AZ_PAIR_ATTR(2, AZ_IN_F32, false); AZ_PAIR_ATTR(2, AZ_IN_POS, false);
+#undef AZ_PAIR_ATTR
+    const char *env = getenv("AZ_NET_PAIR_TILES");     // forces one variant; by default the batch size picks it
+    net->pair_tiles = (env && (atoi(env) == 1 || atoi(env) == 2)) ? atoi(env) : 0;
     return AZ_OK;
 }
 
@@ -594,6 +684,18 @@ void az_net_pair_release(AzNet *net)
     net->pair_stream = net->pair_stream16 = nullptr;
 }
 
+// Profiling hook (not part of the public header, used by tools/net_pair_waits.py): while `d_buf` is non-null, every k_net_pair
+// launch of this context's loaded net runs the one-tile instantiation that writes issuer wait records (PairParams::prof) --
+// (4 + 3 * max_records) int64 per CTA.  It stays set for this context until cleared with a null buffer.
+extern "C" int az_net_pair_profile(az_context *ctx, long long *d_buf, int max_records)
+{
+    AZ_REQUIRE(ctx && ctx->net, AZ_ERR_STATE, "az_net_pair_profile: no weights loaded");
+    AZ_REQUIRE(!d_buf || max_records > 0, AZ_ERR_ARG, "az_net_pair_profile: max_records=%d", max_records);
+    ctx->net->pair_prof = d_buf;
+    ctx->net->pair_prof_max = max_records;
+    return AZ_OK;
+}
+
 int az_net_pair_forward(az_context *ctx, AzNet *net, const void *d_in, int in_kind, int n, float *d_logits, float *d_values, const int *d_count,
                         cudaStream_t stream, int f16)
 {
@@ -612,12 +714,25 @@ int az_net_pair_forward(az_context *ctx, AzNet *net, const void *d_in, int in_ki
     P.f16 = f16;
     static const int relay_mode = getenv("AZ_PAIR_RELAY") ? atoi(getenv("AZ_PAIR_RELAY")) : 2;
     P.relay_mode = relay_mode;
-    const int units = (n + UNIT_BOARDS - 1) / UNIT_BOARDS;
-    int grid = std::min(units, ctx->sm_count * 2);
+    P.prof = net->pair_prof;
+    P.prof_max = net->pair_prof_max;
+    // Two tiles per CTA keep the tensor pipe fed across epilogues, but one CTA per SM only fills the GPU from a full round of
+    // 4 boards per SM on; smaller batches (single trees, latency-bound callers) run one-tile CTAs, two per SM.  The wait
+    // records are taken for the one-tile schedule.
+    const int tiles = P.prof ? 1 : net->pair_tiles ? net->pair_tiles : n >= 4 * ctx->sm_count ? 2 : 1;
+    if (tiles == 2) P.relay_mode = 2;                          // the only relay with per-tile event streams
+    const int unit_boards = tiles == 1 ? PairCfg<1>::UNIT_BOARDS : PairCfg<2>::UNIT_BOARDS;
+    const int units = (n + unit_boards - 1) / unit_boards;
+    int grid = std::min(units, ctx->sm_count * (tiles == 1 ? PairCfg<1>::CTAS_PER_SM : PairCfg<2>::CTAS_PER_SM));
     if (const char *env = getenv("AZ_PAIR_MAX_CTAS")) grid = std::max(2, std::min(grid, atoi(env)));      // experiment knob
     grid = (grid + 1) / 2 * 2;                                  // whole pairs; a surplus CTA runs an all-padding pass
-    if (in_kind == AZ_IN_F32) k_net_pair<AZ_IN_F32><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(P);
-    else k_net_pair<AZ_IN_POS><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(P);
+#define AZ_PAIR_LAUNCH(T, PROF)                                                                                                     \
+    (in_kind == AZ_IN_F32 ? k_net_pair<T, AZ_IN_F32, PROF><<<grid, PairCfg<T>::NUM_THREADS, PairCfg<T>::SMEM_BYTES, stream>>>(P)    \
+                          : k_net_pair<T, AZ_IN_POS, PROF><<<grid, PairCfg<T>::NUM_THREADS, PairCfg<T>::SMEM_BYTES, stream>>>(P))
+    if (P.prof) AZ_PAIR_LAUNCH(1, true);
+    else if (tiles == 1) AZ_PAIR_LAUNCH(1, false);
+    else AZ_PAIR_LAUNCH(2, false);
+#undef AZ_PAIR_LAUNCH
     ctx->launches++;
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;

@@ -10,7 +10,7 @@ t0 = time.perf_counter(); net.load_weights(ctx, network); print("reload %.1f ms"
 lib = _native.lib()
 dev = torch.device("cuda:0")
 stream = torch.cuda.ExternalStream(ctx.stream)
-for B in (256, 1024, 2048, 4096, 16384):
+for B in [int(a) for a in sys.argv[1:]] or (256, 1024, 2048, 4096, 16384):
     feats = (torch.rand(B, 196, device=dev) < 0.3).float()
     logits = torch.empty(B, 833, device=dev); values = torch.empty(B, device=dev)
     torch.cuda.synchronize()

@@ -1295,6 +1295,9 @@ extern "C" float az_trainer_last_step_ms(const az_trainer *t) { return t ? t->la
 //   what = "z" / "act": conv output / activation of `layer` as float [n][7][7][F]      (act: layer 0 = input .. layers = tower output)
 //          "grad_conv": float [9][F][F] of `layer`; "grad_gamma" / "grad_beta" / "gamma" / "beta": float [F] of `layer`;
 //          "grad_heads": float [F*17 + F + 49 + 1]; "moving": float [2][F] of `layer`
+//          "d_h": float [n][7][7][F] (`layer` 0): after a step, the gradient of the loss with respect to layer 0's output.  k_heads
+//          writes the tower output's gradient there, each block's skip and data gradient replace / add to it on the way down,
+//          and layer 0's batch-norm backward reads it without overwriting it (write_g = 0).  After an eval call: unchanged.
 extern "C" int az_trainer_debug_read(az_trainer *t, const char *what, int layer, int n, float *out, size_t count)
 {
     AZ_REQUIRE(t && what && out, AZ_ERR_ARG, "az_trainer_debug_read: null argument");

@@ -117,6 +117,10 @@ class Trainer:
         return float(lib().az_trainer_last_step_ms(self._h))
 
     def debug_read(self, what, layer=0, n=0):
+        """An internal tensor of the last step (test hook; az_train.cu, az_trainer_debug_read).  "z" / "act" / "d_h" take the
+        first n boards as [n, 7, 7, F]: "z" is layer ``layer``'s conv output, "act" its input activation (``layer`` 0 the
+        input features, ``layer`` = layers the tower output), "d_h" the gradient of the loss with respect to layer 0's
+        output after a training step."""
         f = model.Network.FILTERS
         shape = {"z": (n, 7, 7, f), "act": (n, 7, 7, f), "d_h": (n, 7, 7, f), "grad_conv": (3, 3, f, f), "conv": (3, 3, f, f),
                  "grad_gamma": (f,), "grad_beta": (f,), "gamma": (f,), "beta": (f,), "moving": (2, f),

@@ -60,7 +60,6 @@ def test_one_step_matches_fp32_restatement(ctx, blocks, n):
     tile empty (odd batch) and leaves the weight-gradient kernel fewer tiles than ranges; (0, 2) is the smallest legal call: a
     tower of the input conv alone, a batch of two boards."""
     import torch
-    import torch.nn.functional as Fn
     from ataxxzero_b200 import model, trainer
     lr, lam = 0.01, 1e-4
     network = model.Network.random_init(seed=5, blocks=blocks)
@@ -68,24 +67,7 @@ def test_one_step_matches_fp32_restatement(ctx, blocks, n):
     tr = trainer.Trainer(ctx, network, max_batch=64)
     batch = synthetic_batch(n, 1)
     x, pol, val = ref.to_torch_batch(batch, dev)
-    zs, acts = [], []
-
-    def conv_bn(i, inp):
-        z = net.convs[i](inp)
-        zs.append(z)
-        return net.bns[i](z)
-    h = Fn.relu(conv_bn(0, x))
-    acts.append(h)
-    for b in range(blocks):
-        y = Fn.relu(conv_bn(1 + 2 * b, h))
-        acts.append(y)
-        h = Fn.relu(conv_bn(2 + 2 * b, y) + h)
-        acts.append(h)
-    logits = net.policy(h).permute(0, 2, 3, 1).reshape(n, -1)
-    v = torch.tanh(net.value(h).permute(0, 2, 3, 1).reshape(n, 49) @ net.fc_w + net.fc_b)
-    pl = -(pol.reshape(n, -1) * torch.log_softmax(logits, dim=1)).sum(1).mean()
-    vl = ((val - v) ** 2).mean()
-    reg = lam * sum(0.5 * (p ** 2).sum() for p in net.parameters())
+    pl, vl, reg, zs, acts = ref.loss_terms_retained(net, x, pol, val)
     opt.zero_grad()
     (pl + vl + reg).backward()
 
@@ -98,12 +80,16 @@ def test_one_step_matches_fp32_restatement(ctx, blocks, n):
     for p_ in net16.parameters():
         p_.grad = None
     with torch.autocast("cuda", dtype=torch.bfloat16):
-        p16, v16, r16 = ref.loss_terms(net16, x, pol, val)
+        p16, v16, r16, _, acts16 = ref.loss_terms_retained(net16, x, pol, val)
     (p16.float() + v16.float() + r16.float()).backward()
     layers = 1 + 2 * blocks
     for l in range(layers):
         assert rel(tr.debug_read("z", l, n), zs[l].detach().permute(0, 2, 3, 1).cpu().numpy()) < 2e-2, l
         assert rel(tr.debug_read("act", l + 1, n), acts[l].detach().permute(0, 2, 3, 1).cpu().numpy()) < 2e-2, l
+    # d_h after the step: the gradient with respect to layer 0's output (heads, then every data gradient and skip on the way down)
+    d_h, d_ref = tr.debug_read("d_h", 0, n), acts[0].grad.permute(0, 2, 3, 1).cpu().numpy()
+    assert cosine(d_h, d_ref) > 0.98 and abs(np.linalg.norm(d_h) / np.linalg.norm(d_ref) - 1) < 0.03
+    assert rel(d_h, d_ref) < 1.25 * rel(acts16[0].grad.float().permute(0, 2, 3, 1).cpu().numpy(), d_ref) + 1e-3, rel(d_h, d_ref)
     for l in range(layers):
         w = net.convs[l].weight
         g_ref = (w.grad - lam * w).detach().permute(2, 3, 1, 0).cpu().numpy()          # TF order [kx][ky][cin][cout], L2 term removed

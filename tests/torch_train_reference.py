@@ -75,6 +75,37 @@ def loss_terms(net, features, policies, values):
     return policy_loss, value_loss, reg
 
 
+def loss_terms_retained(net, features, policies, values):
+    """loss_terms written out layer by layer, keeping what the native step's debug_read can be compared with:
+    returns (policy_loss, value_loss, reg, zs, acts) where zs[l] is layer l's conv output and acts[l] its output activation
+    (after the residual add and ReLU; acts[-1] is the tower output).  Every acts[l] retains its gradient, so after backward
+    acts[0].grad is the gradient with respect to layer 0's output."""
+    import torch
+    import torch.nn.functional as F
+    zs, acts = [], []
+
+    def conv_bn(i, inp):
+        z = net.convs[i](inp)
+        zs.append(z)
+        return net.bns[i](z)
+
+    def keep(a):
+        a.retain_grad()
+        acts.append(a)
+        return a
+    h = keep(F.relu(conv_bn(0, features)))
+    for b in range((len(net.convs) - 1) // 2):
+        y = keep(F.relu(conv_bn(1 + 2 * b, h)))
+        h = keep(F.relu(conv_bn(2 + 2 * b, y) + h))
+    n = len(features)
+    logits = net.policy(h).permute(0, 2, 3, 1).reshape(n, -1)
+    out = torch.tanh(net.value(h).permute(0, 2, 3, 1).reshape(n, 49) @ net.fc_w + net.fc_b)
+    policy_loss = -(policies.reshape(n, -1) * torch.log_softmax(logits, dim=1)).sum(dim=1).mean()
+    value_loss = ((values - out) ** 2).mean()
+    reg = 0.0001 * sum(0.5 * (p ** 2).sum() for p in net.parameters())
+    return policy_loss, value_loss, reg, zs, acts
+
+
 def to_torch_batch(batch, device):
     import torch
     feats, pol, val = batch

@@ -45,25 +45,8 @@ opt = torch.optim.SGD(net.parameters(), lr=LR, momentum=0.9)
 batch = synthetic_batch(N, 1)
 x, pol, val = ref.to_torch_batch(batch, dev)
 
-# torch forward with intermediates
-zs, acts = [], [x]
-import torch.nn.functional as Fn
-h = x
-def conv_bn(i, inp):
-    z = net.convs[i](inp); z.retain_grad(); zs.append(z)
-    return net.bns[i](z)
-h = Fn.relu(conv_bn(0, x)); acts.append(h)
-for b in range(BLOCKS):
-    y = Fn.relu(conv_bn(1 + 2 * b, h)); acts.append(y)
-    y = conv_bn(2 + 2 * b, y)
-    h = Fn.relu(y + h); acts.append(h)
-h.retain_grad()
-logits = net.policy(h).permute(0, 2, 3, 1).reshape(N, -1)
-v = torch.tanh(net.value(h).permute(0, 2, 3, 1).reshape(N, 49) @ net.fc_w + net.fc_b)
-log_sm = torch.log_softmax(logits, dim=1)
-pl = -(pol.reshape(N, -1) * log_sm).sum(1).mean()
-vl = ((val - v) ** 2).mean()
-reg = 0.0001 * sum(0.5 * (p ** 2).sum() for p in net.parameters())
+# torch forward with intermediates (zs[l] conv output, acts[l] output activation of layer l; acts[0].grad = d loss / d layer 0's output)
+pl, vl, reg, zs, acts = ref.loss_terms_retained(net, x, pol, val)
 opt.zero_grad()
 (pl + vl + reg).backward()
 
@@ -74,9 +57,12 @@ for l in range(L):
     z_ours = tr.debug_read("z", l, N)
     z_ref = zs[l].detach().permute(0, 2, 3, 1).cpu().numpy()
     a_ours = tr.debug_read("act", l + 1, N)
-    a_ref = acts[l + 1].detach().permute(0, 2, 3, 1).cpu().numpy()
+    a_ref = acts[l].detach().permute(0, 2, 3, 1).cpu().numpy()
     print("layer %2d  z rel %.2e  act rel %.2e" % (l, rel(z_ours, z_ref), rel(a_ours, a_ref)))
-print("d_h (tower output grad): n/a after backward (buffer reused)")
+d_ours = tr.debug_read("d_h", 0, N)                                            # after the step: d loss / d (layer 0's output)
+d_ref = acts[0].grad.permute(0, 2, 3, 1).cpu().numpy()
+print("d_h (layer 0 output grad) rel %.2e  cosine %.6f  norm ours %.3e ref %.3e" % (
+    rel(d_ours, d_ref), float(d_ours.ravel() @ d_ref.ravel() / (np.linalg.norm(d_ours) * np.linalg.norm(d_ref))), np.linalg.norm(d_ours), np.linalg.norm(d_ref)))
 lam = 1e-4
 for l in reversed(range(L)):
     g_ours = tr.debug_read("grad_conv", l)

@@ -291,6 +291,15 @@ extern "C" int az_net_forward_counted_dev(az_context *ctx, const void *d_feature
     return net_forward_dev(ctx, d_features, AZ_IN_F32, n, mode, d_logits, d_values, d_count);
 }
 
+// Test hook (not part of the public header): the forward pass exactly as the self-play pool launches it (launch_net in
+// az_pool.cu) -- az_position[] input, board count read from device memory when d_count is non-null, and for a speculative
+// cache pool the softmax numerators, their sequential sums and the values scattered through d_out_map with d_logits null.
+extern "C" int az_net_forward_pool_dev(az_context *ctx, const void *d_pos, int n, const int *d_count, int mode, int tiles, void *d_logits,
+                                       void *d_values, double *d_exps, double *d_totals, const int *d_out_map)
+{
+    return net_forward_dev(ctx, d_pos, AZ_IN_POS, n, mode, d_logits, d_values, d_count, nullptr, tiles, d_exps, d_totals, d_out_map);
+}
+
 extern "C" int az_net_forward_pos_dev(az_context *ctx, const void *d_pos, int n, int mode, void *d_logits, void *d_values)
 {
     return net_forward_dev(ctx, d_pos, AZ_IN_POS, n, mode, d_logits, d_values);

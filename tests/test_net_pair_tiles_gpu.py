@@ -74,6 +74,7 @@ def test_tiles_agree_with_device_count(network):
                 d_count = torch.tensor([count], dtype=torch.int32, device="cuda")
                 logits = torch.full((n, 833), -7.0, device="cuda")
                 values = torch.full((n,), -7.0, device="cuda")
+                torch.cuda.synchronize()          # the fills run on torch's stream, the net on the context's non-blocking stream
                 _native.check(fn(c.handle, C.c_void_p(feats.data_ptr()), n, C.c_void_p(d_count.data_ptr()), mode,
                                  C.c_void_p(logits.data_ptr()), C.c_void_p(values.data_ptr())))
                 c.sync()

@@ -61,7 +61,7 @@ int az_net_tc_forward_sym8(az_context *ctx, AzNet *net, const void *d_in, int in
 int az_net_forward_internal(az_context *ctx, const void *d_in, int in_kind, int n, int mode, float *d_logits, float *d_values,
                             const int *d_count, cudaStream_t stream = nullptr, int tiles = 0, double *d_exps = nullptr,
                             double *d_totals = nullptr, const int *d_out_map = nullptr);
-int az_net_tc_boards_per_round(az_context *ctx, int tiles);   // boards one wave of persistent CTAs evaluates
+int az_net_tc_boards_per_round(az_context *ctx);   // boards one wave of persistent CTAs of the default variant evaluates
 void az_net_tc_release(AzNet *net);
 
 // az_net_pair.cu

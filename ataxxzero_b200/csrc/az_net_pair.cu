@@ -13,9 +13,9 @@
 // second conv of a block accumulates on top of the residual), weights pre-tiled in HBM as the exact shared-memory image
 // of a stage, early release of the first input-channel half.  Roles per CTA: warp 0 = TMA producer (its own half of
 // every stage), warp 1 = MMA issuer in the LEADER (cluster rank 0) / relay in the peer, warps 2-5 = epilogue.
-// The peer's relay thread walks the leader's wait sequence: whenever one of the peer's own barriers completes (weights
-// landed, activations written, input staged) it arrives on the leader's barrier of the same name, so the one issuing
-// thread sees "both halves ready" as a single barrier phase.  tcgen05.commit multicasts completions back to both CTAs.
+// The peer's relay warp (one lane per barrier) forwards completions: whenever one of the peer's own barriers completes
+// (weights landed, activations written, input staged) it arrives on the leader's barrier of the same name, so the one
+// issuing thread sees "both halves ready" as a single barrier phase.  tcgen05.commit multicasts completions back to both CTAs.
 #include "az_net.h"
 #include "az_rules.cuh"
 
@@ -87,12 +87,11 @@ __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes)
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
 // arrive on the barrier at the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t rank, bool relaxed)
+__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t rank)
 {
     uint32_t remote;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(bar), "r"(rank));
-    if (relaxed) asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
-    else asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
+    asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
 {
@@ -203,7 +202,6 @@ struct PairParams {
     const float *fc_w, *fc_b;
     float *logits, *values;
     int f16;
-    int relay_mode;                    // AZ_PAIR_RELAY: 0 one thread / release arrives, 1 one thread / relaxed arrives, 2 one lane per event stream
     long long *prof;                   // issuer wait records (k_net_pair<..., true> only, see az_net_pair_profile)
     int prof_max;                      // records per CTA
 };
@@ -290,54 +288,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PairCfg<TILES>::NUM_
         int my_units = 0;
         for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) ++my_units;
         const int pushes_per_unit = (5 + WIN_KSTEPS_PER_STAGE - 1) / WIN_KSTEPS_PER_STAGE + nl * CHUNKS + 1;
-        if (P.relay_mode == 2) {
-            // every barrier is its own event stream with self-consistent phases: one lane per stream, so that a slow hop on one
-            // of them never delays the others (the weight stages; per tile the two activation parts and the staged input)
-            static_assert(STAGES + TILES * (SPLIT + 1) <= 32, "one relay lane per event stream");
-            const bool relaxed = true;
-            if (lane < STAGES) {
-                const uint32_t total = (uint32_t)my_units * (uint32_t)pushes_per_unit;
-                for (uint32_t it = lane; it < total; it += STAGES) {
-                    mbar_wait(bar(B_FULL + lane), (it / STAGES) & 1);
-                    mbar_arrive_remote(bar(B_FULL + lane), 0, relaxed);
-                }
-            } else if (lane < STAGES + TILES * (SPLIT + 1)) {
-                const int tile = (lane - STAGES) / (SPLIT + 1), k = (lane - STAGES) % (SPLIT + 1);     // k < SPLIT: part k, else input
-                const uint32_t b = tbar(tile, k < SPLIT ? ACT + k : IN);
-                const uint32_t total = (uint32_t)my_units * (uint32_t)(k < SPLIT ? nl + 1 : 1);
-                for (uint32_t e = 0; e < total; ++e) {
-                    mbar_wait(b, e & 1);
-                    mbar_arrive_remote(b, 0, relaxed);
-                }
+        // every barrier is its own event stream with self-consistent phases: one lane per stream, so that a slow hop on one
+        // of them never delays the others (the weight stages; per tile the two activation parts and the staged input)
+        static_assert(STAGES + TILES * (SPLIT + 1) <= 32, "one relay lane per event stream");
+        if (lane < STAGES) {
+            const uint32_t total = (uint32_t)my_units * (uint32_t)pushes_per_unit;
+            for (uint32_t it = lane; it < total; it += STAGES) {
+                mbar_wait(bar(B_FULL + lane), (it / STAGES) & 1);
+                mbar_arrive_remote(bar(B_FULL + lane), 0);
             }
-        } else if (TILES == 1 && elect_one()) {
-            const bool relaxed = P.relay_mode == 1;
-            uint32_t it = 0, in_phase = 0, act_phase = 0;
-            auto relay_stage = [&]() {
-                const int s = it % STAGES;
-                mbar_wait(bar(B_FULL + s), (it / STAGES) & 1);
-                mbar_arrive_remote(bar(B_FULL + s), 0, relaxed);
-                ++it;
-            };
-            for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
-                mbar_wait(tbar(0, IN), in_phase);
-                in_phase ^= 1;
-                mbar_arrive_remote(tbar(0, IN), 0, relaxed);
-                for (int j0 = 0; j0 < 5; j0 += WIN_KSTEPS_PER_STAGE) relay_stage();
-                for (int l = 0; l < nl; ++l) {
-                    for (int part = 0; part < SPLIT; ++part) {
-                        mbar_wait(tbar(0, ACT + part), act_phase);
-                        mbar_arrive_remote(tbar(0, ACT + part), 0, relaxed);
-                        for (int tap = 0; tap < 9; ++tap) relay_stage();
-                    }
-                    act_phase ^= 1;
-                }
-                for (int p = 0; p < SPLIT; ++p) {
-                    mbar_wait(tbar(0, ACT + p), act_phase);
-                    mbar_arrive_remote(tbar(0, ACT + p), 0, relaxed);
-                }
-                act_phase ^= 1;
-                relay_stage();
+        } else if (lane < STAGES + TILES * (SPLIT + 1)) {
+            const int tile = (lane - STAGES) / (SPLIT + 1), k = (lane - STAGES) % (SPLIT + 1);     // k < SPLIT: part k, else input
+            const uint32_t b = tbar(tile, k < SPLIT ? ACT + k : IN);
+            const uint32_t total = (uint32_t)my_units * (uint32_t)(k < SPLIT ? nl + 1 : 1);
+            for (uint32_t e = 0; e < total; ++e) {
+                mbar_wait(b, e & 1);
+                mbar_arrive_remote(b, 0);
             }
         }
     } else if (warp == 1) {
@@ -712,19 +678,15 @@ int az_net_pair_forward(az_context *ctx, AzNet *net, const void *d_in, int in_ki
     P.logits = d_logits;
     P.values = d_values;
     P.f16 = f16;
-    static const int relay_mode = getenv("AZ_PAIR_RELAY") ? atoi(getenv("AZ_PAIR_RELAY")) : 2;
-    P.relay_mode = relay_mode;
     P.prof = net->pair_prof;
     P.prof_max = net->pair_prof_max;
     // Two tiles per CTA keep the tensor pipe fed across epilogues, but one CTA per SM only fills the GPU from a full round of
     // 4 boards per SM on; smaller batches (single trees, latency-bound callers) run one-tile CTAs, two per SM.  The wait
     // records are taken for the one-tile schedule.
     const int tiles = P.prof ? 1 : net->pair_tiles ? net->pair_tiles : n >= 4 * ctx->sm_count ? 2 : 1;
-    if (tiles == 2) P.relay_mode = 2;                          // the only relay with per-tile event streams
     const int unit_boards = tiles == 1 ? PairCfg<1>::UNIT_BOARDS : PairCfg<2>::UNIT_BOARDS;
     const int units = (n + unit_boards - 1) / unit_boards;
     int grid = std::min(units, ctx->sm_count * (tiles == 1 ? PairCfg<1>::CTAS_PER_SM : PairCfg<2>::CTAS_PER_SM));
-    if (const char *env = getenv("AZ_PAIR_MAX_CTAS")) grid = std::max(2, std::min(grid, atoi(env)));      // experiment knob
     grid = (grid + 1) / 2 * 2;                                  // whole pairs; a surplus CTA runs an all-padding pass
 #define AZ_PAIR_LAUNCH(T, PROF)                                                                                                     \
     (in_kind == AZ_IN_F32 ? k_net_pair<T, AZ_IN_F32, PROF><<<grid, PairCfg<T>::NUM_THREADS, PairCfg<T>::SMEM_BYTES, stream>>>(P)    \

@@ -350,7 +350,6 @@ struct TcParams {
     double *totals;                    // [n] their strictly sequential sum (:212-214)
     int f16;                           // operands (weights, activations) are IEEE half instead of bf16: 3 more mantissa bits, 5-bit exponent
     int sym8;                          // 1: `n` positions, each evaluated as the mean over its 8 dihedral images (nn_evals.py:48-62)
-    int experiment;                    // AZ_NET_EXPERIMENT bits: 1 = no weight copies (stale smem), 2 = no tower MMAs.  Wrong results; timing studies only.
 };
 
 // row r of a tile -> board within tile / cell; real rows carry data, the rest are zero padding
@@ -419,7 +418,6 @@ __global__ void __launch_bounds__(Cfg<TILES>::NUM_THREADS, Cfg<TILES>::CTAS_PER_
             auto push = [&](const uint8_t *src, uint32_t bytes) {
                 const int s = it % STAGES;
                 mbar_wait(bar(B_EMPTY + s), ((it / STAGES) & 1) ^ 1);
-                if (P.experiment & 1) { mbar_arrive(bar(B_FULL + s)); ++it; return; }
                 mbar_expect_tx(bar(B_FULL + s), bytes);           // the whole stage: own slice + the peers' slices
                 if (CS == 1) {
                     bulk_g2s(sbase + C::OFF_RING + s * STAGE_BYTES, src, bytes, bar(B_FULL + s));
@@ -916,8 +914,7 @@ static void tc_launch_variant(az_context *ctx, const TcParams &P, int in_kind, i
 {
     using C = Cfg<TILES>;
     const int units = P.sym8 ? n : (n + C::UNIT_BOARDS - 1) / C::UNIT_BOARDS;     // sym8: one work item per position
-    int slots = ctx->sm_count * C::CTAS_PER_SM;
-    if (const char *env = getenv("AZ_NET_MAX_CTAS")) slots = std::max(1, std::min(slots, atoi(env)));     // experiment knob
+    const int slots = ctx->sm_count * C::CTAS_PER_SM;
     int grid = units < slots ? units : slots;
     if (cluster > 1) {
         grid = (grid + cluster - 1) / cluster * cluster;          // whole clusters; surplus CTAs run an all-padding pass
@@ -931,11 +928,10 @@ static void tc_launch_variant(az_context *ctx, const TcParams &P, int in_kind, i
         k_net_tc<TILES, AZ_IN_POS, 1><<<grid, C::NUM_THREADS, C::SMEM_BYTES, stream>>>(P);
 }
 
-int az_net_tc_boards_per_round(az_context *ctx, int tiles)
+int az_net_tc_boards_per_round(az_context *ctx)
 {
-    if (tiles == 0) tiles = ctx->net ? ctx->net->tc_tiles : AZ_NET_TILES_DEFAULT;
-    int slots = tiles == 1 ? ctx->sm_count * Cfg<1>::CTAS_PER_SM : ctx->sm_count * Cfg<2>::CTAS_PER_SM;
-    if (const char *env = getenv("AZ_NET_MAX_CTAS")) slots = std::max(1, std::min(slots, atoi(env)));
+    const int tiles = ctx->net ? ctx->net->tc_tiles : AZ_NET_TILES_DEFAULT;
+    const int slots = tiles == 1 ? ctx->sm_count * Cfg<1>::CTAS_PER_SM : ctx->sm_count * Cfg<2>::CTAS_PER_SM;
     return slots * (tiles == 1 ? Cfg<1>::UNIT_BOARDS : Cfg<2>::UNIT_BOARDS);
 }
 
@@ -966,8 +962,6 @@ static int tc_launch(az_context *ctx, AzNet *net, const void *d_in, int in_kind,
     P.exps = d_exps;
     P.totals = d_totals;
     P.sym8 = sym8;
-    static const int experiment = getenv("AZ_NET_EXPERIMENT") ? atoi(getenv("AZ_NET_EXPERIMENT")) : 0;
-    P.experiment = experiment;
     if (tiles == 1) tc_launch_variant<1>(ctx, P, in_kind, n, stream, net->tc_cluster);
     else tc_launch_variant<2>(ctx, P, in_kind, n, stream, net->tc_cluster);
     ctx->launches++;

@@ -33,40 +33,8 @@ void aztree_launch_debug_exp(const float *d_x, int n, double *d_out, cudaStream_
 void aztree_launch_debug_div(const double *d_in, int n, int puct, double *d_out, cudaStream_t s);
 void aztree_launch_debug_sample(const int32_t *d_visits, int L, int N, uint64_t seed, int n, int32_t *d_out, cudaStream_t s);
 
-// A pool is split into GROUPS of games, each with its own tree memory, request batch and CUDA stream.  One group on the
-// context stream is the default and the measured optimum.  More groups (AZ_POOL_GROUPS=2..4, self-play on the internal net
-// only) let the tree kernel of one group run under the net kernel of another; that overlap is opt-in because it measured
-// SLOWER on B200: a tree kernel that shares SMs with the net kernel's weight stream takes ~2.2x longer (DESIGN.md 3d).
 const int kTicksPerDrain = 32;
 const int kEventPeriod = 1024, kEventWindow = 256;    // CUDA events on the first 256 ticks of every 1024 (run_ticks)
-
-struct Group {
-    PoolDev dev{};
-    cudaStream_t stream = nullptr;
-    bool own_stream = false;
-    int first_game = 0;
-    int slot = 0;                         // req_count slot of the last tick
-    int32_t *d_status = nullptr;
-    float *d_features = nullptr;          // external mode: [G][196]
-    DoneEntry *d_done_snapshot = nullptr; // copy of the done queue being drained
-    uint32_t *d_offsets = nullptr;        // [2G] word offset of every drained record in d_stage
-    uint32_t *d_stage = nullptr;          // finished records packed back to back (k_gather_records)
-    size_t stage_words = 0;
-    // pinned host mirrors
-    int32_t *h_counts = nullptr;          // [0] req_count, [1] busy_count, [2] status, [3] done_count
-    DoneEntry *h_done = nullptr;          // [2G]
-    uint32_t *h_offsets = nullptr;        // [2G]
-    uint32_t *h_stage = nullptr;          // [stage_words]
-    std::vector<Game> h_games;
-    // CUDA events around the tree and the net kernel of EVERY tick between two drains: tree_seconds / net_seconds are sums
-    // of measured launches, not extrapolations
-    // Two sets, used alternately: the set of the batch that just ran is read out AFTER the next batch has been launched,
-    // so the ~100 cudaEventElapsedTime calls never sit between two batches with the GPU idle.
-    std::vector<cudaEvent_t> ev[2];       // [1 + 2 * kTicksPerDrain] each
-    int ev_ticks[2] = {0, 0};             // ticks recorded in the set and not yet read out
-    int ev_cur = 0;
-    unsigned long long *d_timed_evals = nullptr;      // evaluations served by the event-timed net launches (counted on the device)
-};
 
 // Finished games leave the device as packed binary records; turning them into the reference's JSON lines (sorted-key
 // objects, one std::map per ply) costs the host ~0.3 ms per game.  A writer thread does that, so the thread that launches
@@ -90,13 +58,33 @@ struct RecordWriter {
     void run();
 };
 
+// Every kernel and copy of a pool runs on the context stream.
 struct az_pool {
     az_context *ctx = nullptr;
     RecordWriter writer;
     az_pool_config cfg{};
-    std::vector<Group> groups;
-    std::vector<int> group_size;          // games per group (sums to cfg.games)
-    int net_tiles = 0;                    // net kernel variant used by this pool (0 = context default)
+    PoolDev dev{};
+    int slot = 0;                         // req_count slot of the last tick
+    int32_t *d_status = nullptr;
+    float *d_features = nullptr;          // external mode: [G][196]
+    DoneEntry *d_done_snapshot = nullptr; // copy of the done queue being drained
+    uint32_t *d_offsets = nullptr;        // [2G] word offset of every drained record in d_stage
+    uint32_t *d_stage = nullptr;          // finished records packed back to back (k_gather_records)
+    size_t stage_words = 0;
+    // pinned host mirrors
+    int32_t *h_counts = nullptr;          // [0] req_count, [1] busy_count, [2] status, [3] done_count
+    DoneEntry *h_done = nullptr;          // [2G]
+    uint32_t *h_offsets = nullptr;        // [2G]
+    uint32_t *h_stage = nullptr;          // [stage_words]
+    std::vector<Game> h_games;
+    // CUDA events around the tree and the net kernel of EVERY tick between two drains: tree_seconds / net_seconds are sums
+    // of measured launches, not extrapolations
+    // Two sets, used alternately: the set of the batch that just ran is read out AFTER the next batch has been launched,
+    // so the ~100 cudaEventElapsedTime calls never sit between two batches with the GPU idle.
+    std::vector<cudaEvent_t> ev[2];       // [1 + 2 * kTicksPerDrain] each
+    int ev_ticks[2] = {0, 0};             // ticks recorded in the set and not yet read out
+    int ev_cur = 0;
+    unsigned long long *d_timed_evals = nullptr;      // evaluations served by the event-timed net launches (counted on the device)
     int pending_requests = 0;             // external mode: requests handed out by collect()
     uint64_t ticks = 0, launches = 0;
     double net_seconds = 0.0, tree_seconds = 0.0;     // sums over every launch of the self-play loop (CUDA events)
@@ -105,13 +93,6 @@ struct az_pool {
     uint64_t timed_evals_host = 0;                    // evaluations of the timed launches that closed a batch (counted after its sync)
     uint64_t written_games = 0, written_positions = 0, d2h_bytes = 0;
 
-    Group &group_of(int game, int *local)
-    {
-        size_t gi = 0;
-        while (gi + 1 < groups.size() && game >= groups[gi + 1].first_game) ++gi;
-        *local = game - groups[gi].first_game;
-        return groups[gi];
-    }
     int G() const { return cfg.games; }
 };
 
@@ -129,53 +110,43 @@ int dev_alloc(T **p, size_t count, bool zero = true)
 
 const char *kErrNames[] = {"", "node pool exhausted", "selection path longer than 1024 plies", ">= 256 legal moves"};
 
-int sync_all(az_pool *pool)
-{
-    AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
-    for (Group &g : pool->groups)
-        if (g.own_stream) AZ_CUDA(cudaStreamSynchronize(g.stream));
-    return AZ_OK;
-}
-
 int check_game_errors(az_pool *pool)
 {
     // called after a sync: any game in ST_ERROR turns into AZ_ERR_CAPACITY
-    for (Group &grp : pool->groups) {
-        AZ_CUDA(cudaMemcpy(grp.h_games.data(), grp.dev.games, sizeof(Game) * grp.dev.G, cudaMemcpyDeviceToHost));
-        for (int g = 0; g < grp.dev.G; ++g)
-            if (grp.h_games[g].status == ST_ERROR)
-                return az_fail(AZ_ERR_CAPACITY, "game %d: %s", grp.first_game + g, kErrNames[std::min(std::max(grp.h_games[g].error, 0), 3)]);
-    }
+    AZ_CUDA(cudaMemcpy(pool->h_games.data(), pool->dev.games, sizeof(Game) * pool->dev.G, cudaMemcpyDeviceToHost));
+    for (int g = 0; g < pool->dev.G; ++g)
+        if (pool->h_games[g].status == ST_ERROR)
+            return az_fail(AZ_ERR_CAPACITY, "game %d: %s", g, kErrNames[std::min(std::max(pool->h_games[g].error, 0), 3)]);
     return AZ_OK;
 }
 
 // ---- one tick: (previous evaluations ->) tree kernel -> requests ----
-int launch_tree(az_pool *pool, Group &grp, bool consume = true)
+int launch_tree(az_pool *pool, bool consume = true)
 {
-    cudaStream_t s = grp.stream;
-    if (consume) grp.slot = (grp.slot + 1) % 3;          // the kernel itself zeroes the slot after this one
-    else AZ_CUDA(cudaMemsetAsync(grp.dev.req_count + 2 * grp.slot + 1, 0, sizeof(int32_t), s));   // top-up: same slot, fresh busy count
-    grp.dev.consume = consume ? 1 : 0;
-    grp.dev.tick_slot = grp.slot;
-    grp.dev.tick_id++;
-    aztree_launch_tick(grp.dev, s);
-    const int kernels = grp.dev.cache_tag ? 1 : 2;        // + k_order_requests
+    cudaStream_t s = pool->ctx->stream;
+    if (consume) pool->slot = (pool->slot + 1) % 3;      // the kernel itself zeroes the slot after this one
+    else AZ_CUDA(cudaMemsetAsync(pool->dev.req_count + 2 * pool->slot + 1, 0, sizeof(int32_t), s));   // top-up: same slot, fresh busy count
+    pool->dev.consume = consume ? 1 : 0;
+    pool->dev.tick_slot = pool->slot;
+    pool->dev.tick_id++;
+    aztree_launch_tick(pool->dev, s);
+    const int kernels = pool->dev.cache_tag ? 1 : 2;      // + k_order_requests
     pool->launches += kernels;
     pool->ctx->launches += kernels;
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;
 }
 
-int launch_net(az_pool *pool, Group &grp)
+int launch_net(az_pool *pool)
 {
-    const PoolDev &D = grp.dev;
+    const PoolDev &D = pool->dev;
     int rc;
     if (D.cache_tag)      // speculative search pool: every evaluation of the batch lands in its cache entry
         rc = az_net_forward_internal(pool->ctx, D.req_pos, AZ_IN_POS, D.req_cap, pool->cfg.eval_mode, nullptr, D.cache_val,
-                                     D.req_count + 2 * grp.slot, grp.stream, pool->net_tiles, D.cache_exps, D.cache_tot, D.req_out);
+                                     D.req_count + 2 * pool->slot, pool->ctx->stream, 0, D.cache_exps, D.cache_tot, D.req_out);
     else
         rc = az_net_forward_internal(pool->ctx, D.req_pos, AZ_IN_POS, D.cap, pool->cfg.eval_mode, D.logits, D.values,
-                                     D.req_count + 2 * grp.slot, grp.stream, pool->net_tiles);
+                                     D.req_count + 2 * pool->slot, pool->ctx->stream);
     pool->launches++;
     return rc;
 }
@@ -285,42 +256,42 @@ void RecordWriter::shutdown()
 
 namespace {
 
-// Copy out a group's finished games, append them to `out` (may be null: records are dropped), release the buffers.
+// Copy out the pool's finished games, append them to `out` (may be null: records are dropped), release the buffers.
 // The records are packed into one staging buffer on the device and cross PCIe in ONE copy per drain.
-int drain_finished(az_pool *pool, Group &grp, FILE *out, int64_t *games_written, bool copy_payload = true)
+int drain_finished(az_pool *pool, FILE *out, int64_t *games_written, bool copy_payload = true)
 {
-    cudaStream_t s = grp.stream;
-    AZ_CUDA(cudaMemcpyAsync(grp.h_counts + 3, grp.dev.done_count, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    cudaStream_t s = pool->ctx->stream;
+    AZ_CUDA(cudaMemcpyAsync(pool->h_counts + 3, pool->dev.done_count, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     AZ_CUDA(cudaStreamSynchronize(s));
-    const int n = grp.h_counts[3];
+    const int n = pool->h_counts[3];
     if (n == 0) return AZ_OK;
-    AZ_CUDA(cudaMemcpyAsync(grp.h_done, grp.dev.done, sizeof(DoneEntry) * n, cudaMemcpyDeviceToHost, s));
-    AZ_CUDA(cudaMemcpyAsync(grp.d_done_snapshot, grp.dev.done, sizeof(DoneEntry) * n, cudaMemcpyDeviceToDevice, s));
-    AZ_CUDA(cudaMemsetAsync(grp.dev.done_count, 0, sizeof(int32_t), s));
+    AZ_CUDA(cudaMemcpyAsync(pool->h_done, pool->dev.done, sizeof(DoneEntry) * n, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaMemcpyAsync(pool->d_done_snapshot, pool->dev.done, sizeof(DoneEntry) * n, cudaMemcpyDeviceToDevice, s));
+    AZ_CUDA(cudaMemsetAsync(pool->dev.done_count, 0, sizeof(int32_t), s));
     AZ_CUDA(cudaStreamSynchronize(s));
     if (copy_payload) {
         for (int first = 0; first < n;) {                 // normally one pass; more only if a drain exceeds the staging buffer
             size_t words = 0;
             int last = first;
-            while (last < n && words + (size_t)grp.h_done[last].words <= grp.stage_words) {
-                grp.h_offsets[last] = (uint32_t)words;
-                words += (size_t)grp.h_done[last].words;
+            while (last < n && words + (size_t)pool->h_done[last].words <= pool->stage_words) {
+                pool->h_offsets[last] = (uint32_t)words;
+                words += (size_t)pool->h_done[last].words;
                 ++last;
             }
-            if (last == first) return az_fail(AZ_ERR_CAPACITY, "record of %d words exceeds the staging buffer", grp.h_done[first].words);
+            if (last == first) return az_fail(AZ_ERR_CAPACITY, "record of %d words exceeds the staging buffer", pool->h_done[first].words);
             const int m = last - first;
-            AZ_CUDA(cudaMemcpyAsync(grp.d_offsets, grp.h_offsets + first, sizeof(uint32_t) * m, cudaMemcpyHostToDevice, s));
-            aztree_launch_gather(grp.dev, grp.d_done_snapshot + first, grp.d_offsets, m, grp.d_stage, s);
+            AZ_CUDA(cudaMemcpyAsync(pool->d_offsets, pool->h_offsets + first, sizeof(uint32_t) * m, cudaMemcpyHostToDevice, s));
+            aztree_launch_gather(pool->dev, pool->d_done_snapshot + first, pool->d_offsets, m, pool->d_stage, s);
             pool->launches++;
-            AZ_CUDA(cudaMemcpyAsync(grp.h_stage, grp.d_stage, sizeof(uint32_t) * words, cudaMemcpyDeviceToHost, s));
+            AZ_CUDA(cudaMemcpyAsync(pool->h_stage, pool->d_stage, sizeof(uint32_t) * words, cudaMemcpyDeviceToHost, s));
             AZ_CUDA(cudaStreamSynchronize(s));
             pool->d2h_bytes += sizeof(uint32_t) * (uint64_t)words;
             if (out) {                                    // JSON and file I/O happen on the writer thread
                 RecordJob job;
                 job.out = out;
-                job.words.assign(grp.h_stage, grp.h_stage + words);
-                job.done.assign(grp.h_done + first, grp.h_done + last);
-                job.offsets.assign(grp.h_offsets + first, grp.h_offsets + last);
+                job.words.assign(pool->h_stage, pool->h_stage + words);
+                job.done.assign(pool->h_done + first, pool->h_done + last);
+                job.offsets.assign(pool->h_offsets + first, pool->h_offsets + last);
                 pool->writer.push(std::move(job));
             }
             first = last;
@@ -328,31 +299,29 @@ int drain_finished(az_pool *pool, Group &grp, FILE *out, int64_t *games_written,
     }
     for (int i = 0; i < n; ++i) {
         pool->written_games++;
-        pool->written_positions += grp.h_done[i].plies;
+        pool->written_positions += pool->h_done[i].plies;
         if (games_written) (*games_written)++;
     }
-    aztree_launch_release(grp.dev, grp.d_done_snapshot, n, s);
+    aztree_launch_release(pool->dev, pool->d_done_snapshot, n, s);
     pool->launches++;
     return AZ_OK;
 }
 
-void free_group(Group &grp)
+void free_buffers(az_pool *pool)
 {
-    PoolDev &D = grp.dev;
+    PoolDev &D = pool->dev;
     void *ptrs[] = {D.nodes, D.games, D.path, D.gstack, D.req_pos, D.req_game, D.req_stage, D.req_mark, D.req_count, D.logits, D.values, D.cache_tag,
                     D.cache_exps, D.cache_tot, D.cache_val, D.req_out, D.records,
-                    D.done, D.done_count, grp.d_done_snapshot, grp.d_status, grp.d_timed_evals, grp.d_features, grp.d_offsets, grp.d_stage};
+                    D.done, D.done_count, pool->d_done_snapshot, pool->d_status, pool->d_timed_evals, pool->d_features, pool->d_offsets, pool->d_stage};
     for (void *p : ptrs)
         if (p) cudaFree(p);
-    if (grp.h_counts) cudaFreeHost(grp.h_counts);
-    if (grp.h_done) cudaFreeHost(grp.h_done);
-    if (grp.h_offsets) cudaFreeHost(grp.h_offsets);
-    if (grp.h_stage) cudaFreeHost(grp.h_stage);
-    for (auto &set : grp.ev)
+    if (pool->h_counts) cudaFreeHost(pool->h_counts);
+    if (pool->h_done) cudaFreeHost(pool->h_done);
+    if (pool->h_offsets) cudaFreeHost(pool->h_offsets);
+    if (pool->h_stage) cudaFreeHost(pool->h_stage);
+    for (auto &set : pool->ev)
       for (auto &e : set)
         if (e) cudaEventDestroy(e);
-    if (grp.own_stream && grp.stream) cudaStreamDestroy(grp.stream);
-    grp = Group();
 }
 
 bool valid_position(const az_position &r)
@@ -387,47 +356,7 @@ extern "C" int az_pool_create(az_context *ctx, const az_pool_config *cfg, az_poo
     if (pool->cfg.steps_per_tick <= 0) pool->cfg.steps_per_tick = 8;
     AZ_REQUIRE(pool->cfg.node_capacity < (1 << 24), AZ_ERR_ARG, "az_pool_create: node_capacity too large");
 
-    // Self-play on the internal tensor-core net: two groups that take turns on the net kernel (see Group).  The
-    // 2-tile net variant (one CTA per SM) is used there because it leaves room for the tree blocks on every SM.
     const bool tensor_net = cfg->eval_mode == AZ_NET_BF16 || cfg->eval_mode == AZ_NET_F16;
-    const bool pipelined = cfg->auto_play && tensor_net;
-    int n_groups = 1;
-    if (pipelined) {
-        const char *env = getenv("AZ_POOL_GROUPS");
-        const int round1 = az_net_tc_boards_per_round(ctx, 0);
-        // Measured on B200 (2048 games x 800 visits): a tree kernel that shares the SMs with the net kernel runs ~2.2x
-        // slower (the net streams ~12 TB/s of weights out of L2), which eats the overlap: 2 groups give 2.50 M
-        // evaluations/s against 2.69 M for one group with whole-round request batches.  So: opt-in (AZ_POOL_GROUPS=2).
-        (void)round1;
-        n_groups = env ? std::max(1, std::min(atoi(env), 4)) : 1;
-        n_groups = std::min(n_groups, cfg->games);
-        const char *tiles_env = getenv("AZ_POOL_NET_TILES");
-        if (tiles_env) pool->net_tiles = atoi(tiles_env) == 1 ? 1 : atoi(tiles_env) == 2 ? 2 : 0;
-    }
-    // group sizes: equal shares, or AZ_POOL_SPLIT="1536,512" (an asymmetric split lets the small group's net launch
-    // hide inside the big group's tree kernel and vice versa)
-    pool->group_size.assign(n_groups, 0);
-    for (int gi = 0; gi < n_groups; ++gi) pool->group_size[gi] = cfg->games / n_groups + (gi < cfg->games % n_groups ? 1 : 0);
-    if (const char *split = pipelined ? getenv("AZ_POOL_SPLIT") : nullptr) {
-        std::vector<int> sizes;
-        int total = 0;
-        for (const char *p = split; *p;) {
-            char *end = nullptr;
-            const long v = strtol(p, &end, 10);
-            if (end == p || v <= 0) { sizes.clear(); break; }
-            sizes.push_back((int)v);
-            total += (int)v;
-            p = *end == ',' ? end + 1 : end;
-        }
-        if (sizes.empty() || total != cfg->games || sizes.size() > 4) {
-            delete pool;
-            return az_fail(AZ_ERR_ARG, "az_pool_create: AZ_POOL_SPLIT='%s' must list 1..4 positive group sizes that sum to games=%d", split, cfg->games);
-        }
-        pool->group_size = sizes;
-        n_groups = (int)sizes.size();
-    }
-    pool->groups.resize(n_groups);
-
     size_t free_b = 0, total_b = 0;
     AZ_CUDA(cudaMemGetInfo(&free_b, &total_b));
     const uint32_t rec_cap_words = cfg->auto_play ? (uint32_t)pool->cfg.max_plies * kRecWordsPerPly : 16;
@@ -439,108 +368,93 @@ extern "C" int az_pool_create(az_context *ctx, const az_pool_config *cfg, az_poo
             return az_fail(AZ_ERR_CAPACITY, "az_pool_create: needs %.1f GiB of HBM, %.1f GiB free", need / 1073741824.0, free_b / 1073741824.0);
         }
     }
-    int rc = 0;
-    for (int gi = 0; gi < n_groups && rc == 0; ++gi) {
-        Group &grp = pool->groups[gi];
-        grp.first_game = gi == 0 ? 0 : pool->groups[gi - 1].first_game + pool->group_size[gi - 1];
-        PoolDev &D = grp.dev;
-        D.G = pool->group_size[gi];
-        D.C = pool->cfg.node_capacity;
-        D.visits = cfg->visits;
-        D.max_plies = pool->cfg.max_plies;
-        D.noise = cfg->noise ? 1 : 0;
-        D.auto_play = cfg->auto_play ? 1 : 0;
-        D.steps_per_tick = pool->cfg.steps_per_tick;
-        D.game_base = grp.first_game;
-        // evaluations per tick: a whole number of rounds of the net kernel's persistent CTAs, so its last round is
-        // never half empty; later requests are re-queued.  Self-play only (search pools serve every request).
-        D.cap = D.G;
-        if (pipelined) {
-            const int round = az_net_tc_boards_per_round(ctx, pool->net_tiles);
-            const char *env = getenv("AZ_REQ_CAP");            // one value, or one per group ("1184,444")
-            for (int k = 0; env && k < gi; ++k) {
-                const char *comma = strchr(env, ',');
-                if (!comma) break;
-                env = comma + 1;
-            }
-            if (env) D.cap = atoi(env) > 0 ? std::min(atoi(env), D.G) : D.G;
-            else if (D.G >= round) D.cap = D.G / round * round;
-        }
-        // the level budget trims the tail of a tick over thousands of games; a handful of trees has no tail to trim, and a
-        // suspended descent would cost it a whole (empty) net launch
-        // No default budget is in clock cycles: how far a game gets would then depend on timing, and the same seed would
-        // not replay the same games (AZ_TICK_CYCLES sets one for experiments).
-        D.levels_per_tick = getenv("AZ_LEVELS_PER_TICK") ? atoi(getenv("AZ_LEVELS_PER_TICK")) : (cfg->games < 64 ? (1 << 20) : 48);
-        D.seed = cfg->seed;
-        D.tick_cycles = getenv("AZ_TICK_CYCLES") ? atoi(getenv("AZ_TICK_CYCLES")) : 0;
-        D.prefetch = getenv("AZ_TREE_PREFETCH") ? atoi(getenv("AZ_TREE_PREFETCH")) : 8;
-        D.force_slow = getenv("AZ_TREE_FORCE_SLOW") ? atoi(getenv("AZ_TREE_FORCE_SLOW")) : 0;
-        D.one_random_move = (cfg->auto_play && cfg->one_random_move) ? 1 : 0;
-        D.rec_cap_words = rec_cap_words;
-        const size_t G = (size_t)D.G;
-        rc |= dev_alloc(&D.nodes, G * D.C * kNodeStride, false);
-        rc |= dev_alloc(&D.games, G);
-        rc |= dev_alloc(&D.path, G * kMaxPath, false);
-        rc |= dev_alloc(&D.gstack, G * D.C, false);
-        rc |= dev_alloc(&D.req_pos, G);
-        rc |= dev_alloc(&D.req_game, G);
-        rc |= dev_alloc(&D.req_stage, G);
-        rc |= dev_alloc(&D.req_mark, G);          // zero: no tick 0 is ever launched
-        rc |= dev_alloc(&D.req_count, 8);
-        rc |= dev_alloc(&D.logits, G * AZ_LOGITS);
-        rc |= dev_alloc(&D.values, G);
-        const int spec_k = (tensor_net && !cfg->auto_play) ? std::min(std::max(cfg->speculate, 0), 64) : 0;
-        if (spec_k > 0) {
-            // speculative evaluation: a per-game cache of evaluations + a request batch that can hold the extra requests
-            int entries = 1024;
-            while (entries < 2 * pool->cfg.node_capacity && entries < (1 << 18)) entries *= 2;    // 6.7 KB per entry
-            D.cache_entries = entries;
-            D.spec_k = spec_k;
-            D.req_cap = std::max(2 * az_net_tc_boards_per_round(ctx, pool->net_tiles), (int)G * (1 + spec_k));
-            const size_t total = G * (size_t)entries + 1;        // + the trash entry
-            rc |= dev_alloc(&D.cache_tag, total);
-            rc |= dev_alloc(&D.cache_exps, total * AZ_LOGITS, false);
-            rc |= dev_alloc(&D.cache_tot, total, false);
-            rc |= dev_alloc(&D.cache_val, total, false);
-            rc |= dev_alloc(&D.req_out, (size_t)D.req_cap);
-            cudaFree(D.req_pos);
-            D.req_pos = nullptr;
-            rc |= dev_alloc(&D.req_pos, (size_t)std::max<int>(D.req_cap, (int)G));
-        }
-        rc |= dev_alloc(&D.records, G * 2 * D.rec_cap_words, false);
-        rc |= dev_alloc(&D.done, 2 * G);
-        rc |= dev_alloc(&D.done_count, 1);
-        rc |= dev_alloc(&grp.d_done_snapshot, 2 * G);
-        rc |= dev_alloc(&grp.d_offsets, 2 * G);
-        // staging for one drain: every game can hand over at most its two record buffers; in practice a drain carries a few
-        // dozen games, so the buffer is sized for 64 full-length records (a larger drain is fetched in several passes)
-        grp.stage_words = (size_t)D.rec_cap_words * (cfg->auto_play ? std::min<size_t>(2 * G, 64) : 1);
-        rc |= dev_alloc(&grp.d_stage, grp.stage_words, false);
-        rc |= dev_alloc(&grp.d_status, 4);
-        rc |= dev_alloc(&grp.d_timed_evals, 1);
-        rc |= dev_alloc(&grp.d_features, G * AZ_FEATURES);
-        if (rc) break;
-        if (cudaMallocHost(&grp.h_counts, 16 * sizeof(int32_t)) != cudaSuccess || cudaMallocHost(&grp.h_done, sizeof(DoneEntry) * 2 * G) != cudaSuccess ||
-            cudaMallocHost(&grp.h_offsets, sizeof(uint32_t) * 2 * G) != cudaSuccess ||
-            cudaMallocHost(&grp.h_stage, sizeof(uint32_t) * grp.stage_words) != cudaSuccess) { rc = az_fail(AZ_ERR_CUDA, "az_pool_create: pinned host alloc"); break; }
-        grp.h_games.resize(G);
-        for (auto &set : grp.ev) {
-            set.assign(1 + 2 * kTicksPerDrain, nullptr);
-            for (auto &e : set)
-                if (cudaEventCreate(&e) != cudaSuccess) rc = az_fail(AZ_ERR_CUDA, "az_pool_create: event");
-        }
-        if (n_groups > 1) {
-            if (cudaStreamCreateWithFlags(&grp.stream, cudaStreamNonBlocking) != cudaSuccess) { rc = az_fail(AZ_ERR_CUDA, "az_pool_create: stream"); break; }
-            grp.own_stream = true;
-        } else {
-            grp.stream = ctx->stream;
-        }
-        if (getenv("AZ_POOL_PROFILE")) rc |= dev_alloc(&D.prof, G * 16);
-        aztree_launch_init_all(D, start, grp.stream);
-        pool->launches++;
+    PoolDev &D = pool->dev;
+    D.G = cfg->games;
+    D.C = pool->cfg.node_capacity;
+    D.visits = cfg->visits;
+    D.max_plies = pool->cfg.max_plies;
+    D.noise = cfg->noise ? 1 : 0;
+    D.auto_play = cfg->auto_play ? 1 : 0;
+    D.steps_per_tick = pool->cfg.steps_per_tick;
+    // evaluations per tick: a whole number of rounds of the net kernel's persistent CTAs, so its last round is
+    // never half empty; later requests are re-queued.  Self-play on the tensor-core net only (search pools serve every
+    // request).  AZ_REQ_CAP=<n> sets the cap, 0 serves every request.
+    D.cap = D.G;
+    if (cfg->auto_play && tensor_net) {
+        const int round = az_net_tc_boards_per_round(ctx);
+        if (const char *env = getenv("AZ_REQ_CAP")) D.cap = atoi(env) > 0 ? std::min(atoi(env), D.G) : D.G;
+        else if (D.G >= round) D.cap = D.G / round * round;
     }
-    if (rc) { az_pool_destroy(pool); return rc ? rc : AZ_ERR_CUDA; }
-    if ((rc = sync_all(pool))) { az_pool_destroy(pool); return rc; }
+    // the level budget trims the tail of a tick over thousands of games; a handful of trees has no tail to trim, and a
+    // suspended descent would cost it a whole (empty) net launch
+    // The budget is in levels, not in clock cycles: how far a game gets would then depend on timing, and the same seed
+    // would not replay the same games.
+    D.levels_per_tick = getenv("AZ_LEVELS_PER_TICK") ? atoi(getenv("AZ_LEVELS_PER_TICK")) : (cfg->games < 64 ? (1 << 20) : 48);
+    D.seed = cfg->seed;
+    D.prefetch = getenv("AZ_TREE_PREFETCH") ? atoi(getenv("AZ_TREE_PREFETCH")) : 8;
+    D.force_slow = getenv("AZ_TREE_FORCE_SLOW") ? atoi(getenv("AZ_TREE_FORCE_SLOW")) : 0;
+    D.one_random_move = (cfg->auto_play && cfg->one_random_move) ? 1 : 0;
+    D.rec_cap_words = rec_cap_words;
+    const size_t G = (size_t)D.G;
+    int rc = 0;
+    rc |= dev_alloc(&D.nodes, G * D.C * kNodeStride, false);
+    rc |= dev_alloc(&D.games, G);
+    rc |= dev_alloc(&D.path, G * kMaxPath, false);
+    rc |= dev_alloc(&D.gstack, G * D.C, false);
+    rc |= dev_alloc(&D.req_pos, G);
+    rc |= dev_alloc(&D.req_game, G);
+    rc |= dev_alloc(&D.req_stage, G);
+    rc |= dev_alloc(&D.req_mark, G);          // zero: no tick 0 is ever launched
+    rc |= dev_alloc(&D.req_count, 8);
+    rc |= dev_alloc(&D.logits, G * AZ_LOGITS);
+    rc |= dev_alloc(&D.values, G);
+    const int spec_k = (tensor_net && !cfg->auto_play) ? std::min(std::max(cfg->speculate, 0), 64) : 0;
+    if (spec_k > 0) {
+        // speculative evaluation: a per-game cache of evaluations + a request batch that can hold the extra requests
+        int entries = 1024;
+        while (entries < 2 * pool->cfg.node_capacity && entries < (1 << 18)) entries *= 2;    // 6.7 KB per entry
+        D.cache_entries = entries;
+        D.spec_k = spec_k;
+        D.req_cap = std::max(2 * az_net_tc_boards_per_round(ctx), (int)G * (1 + spec_k));
+        const size_t total = G * (size_t)entries + 1;        // + the trash entry
+        rc |= dev_alloc(&D.cache_tag, total);
+        rc |= dev_alloc(&D.cache_exps, total * AZ_LOGITS, false);
+        rc |= dev_alloc(&D.cache_tot, total, false);
+        rc |= dev_alloc(&D.cache_val, total, false);
+        rc |= dev_alloc(&D.req_out, (size_t)D.req_cap);
+        cudaFree(D.req_pos);
+        D.req_pos = nullptr;
+        rc |= dev_alloc(&D.req_pos, (size_t)std::max<int>(D.req_cap, (int)G));
+    }
+    rc |= dev_alloc(&D.records, G * 2 * D.rec_cap_words, false);
+    rc |= dev_alloc(&D.done, 2 * G);
+    rc |= dev_alloc(&D.done_count, 1);
+    rc |= dev_alloc(&pool->d_done_snapshot, 2 * G);
+    rc |= dev_alloc(&pool->d_offsets, 2 * G);
+    // staging for one drain: every game can hand over at most its two record buffers; in practice a drain carries a few
+    // dozen games, so the buffer is sized for 64 full-length records (a larger drain is fetched in several passes)
+    pool->stage_words = (size_t)D.rec_cap_words * (cfg->auto_play ? std::min<size_t>(2 * G, 64) : 1);
+    rc |= dev_alloc(&pool->d_stage, pool->stage_words, false);
+    rc |= dev_alloc(&pool->d_status, 4);
+    rc |= dev_alloc(&pool->d_timed_evals, 1);
+    rc |= dev_alloc(&pool->d_features, G * AZ_FEATURES);
+    if (rc == 0 && (cudaMallocHost(&pool->h_counts, 16 * sizeof(int32_t)) != cudaSuccess ||
+                    cudaMallocHost(&pool->h_done, sizeof(DoneEntry) * 2 * G) != cudaSuccess ||
+                    cudaMallocHost(&pool->h_offsets, sizeof(uint32_t) * 2 * G) != cudaSuccess ||
+                    cudaMallocHost(&pool->h_stage, sizeof(uint32_t) * pool->stage_words) != cudaSuccess))
+        rc = az_fail(AZ_ERR_CUDA, "az_pool_create: pinned host alloc");
+    pool->h_games.resize(G);
+    for (auto &set : pool->ev) {
+        set.assign(1 + 2 * kTicksPerDrain, nullptr);
+        for (auto &e : set)
+            if (cudaEventCreate(&e) != cudaSuccess) rc = az_fail(AZ_ERR_CUDA, "az_pool_create: event");
+    }
+    if (getenv("AZ_POOL_PROFILE")) rc |= dev_alloc(&D.prof, G * 16);
+    if (rc) { az_pool_destroy(pool); return rc; }
+    aztree_launch_init_all(D, start, ctx->stream);
+    pool->launches++;
+    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) { az_pool_destroy(pool); return az_fail(AZ_ERR_CUDA, "az_pool_create: %s", cudaGetErrorString(e)); }
     AZ_CUDA(cudaGetLastError());
     if ((rc = check_game_errors(pool))) { az_pool_destroy(pool); return rc; }
     *out = pool;
@@ -553,93 +467,87 @@ extern "C" void az_pool_destroy(az_pool *pool)
     cudaStreamSynchronize(pool->ctx->stream);
     pool->writer.flush();
     pool->writer.shutdown();
-    for (Group &grp : pool->groups) {
-        if (grp.stream) cudaStreamSynchronize(grp.stream);
-        if (grp.dev.prof) {              // per-phase cycles, accumulated over every tick: mean and worst game
-            std::vector<unsigned long long> h((size_t)grp.dev.G * 16);
-            cudaMemcpy(h.data(), grp.dev.prof, h.size() * 8, cudaMemcpyDeviceToHost);
-            const char *names[6] = {"populate", "backup", "descent", "expand", "make_move", "total"};
-            for (int ph = 0; ph < 6; ++ph) {
-                double sum = 0, mx = 0;
-                for (int g = 0; g < grp.dev.G; ++g) { sum += (double)h[(size_t)g * 16 + ph]; mx = std::max(mx, (double)h[(size_t)g * 16 + ph]); }
-                fprintf(stderr, "[az_pool profile] %-9s mean %.1f kcycles/tick/game, worst game %.1f kcycles/tick (%llu ticks)\n", names[ph],
-                        sum / grp.dev.G / std::max<uint64_t>(pool->ticks, 1) / 1e3, mx / std::max<uint64_t>(pool->ticks, 1) / 1e3,
-                        (unsigned long long)pool->ticks);
-            }
-            // the last tick on the wall clock: when did each game start and finish inside the kernel?
-            std::vector<double> start, finish;
-            unsigned long long t0 = ~0ull;
-            for (int g = 0; g < grp.dev.G; ++g)
-                if (h[(size_t)g * 16 + 6]) t0 = std::min(t0, h[(size_t)g * 16 + 6]);
-            std::vector<std::pair<double, int>> order;
-            for (int g = 0; g < grp.dev.G; ++g)
-                if (h[(size_t)g * 16 + 6]) {
-                    start.push_back((double)(h[(size_t)g * 16 + 6] - t0) * 1e-3);
-                    finish.push_back((double)(h[(size_t)g * 16 + 7] - t0) * 1e-3);
-                    order.push_back({finish.back(), g});
-                }
-            // what the games of each finish-time band did in that tick (cycles per phase, steps, tree levels)
-            std::sort(order.begin(), order.end());
-            const double bands[6] = {0.0, 0.25, 0.5, 0.75, 0.9, 0.97};
-            for (int b = 0; b < 6 && !order.empty(); ++b) {
-                const size_t lo = (size_t)(bands[b] * order.size()), hi = b == 5 ? order.size() : (size_t)(bands[b + 1] * order.size());
-                if (hi <= lo) continue;                    // pools of a few games: not every band has one
-                double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, waiting = 0;
-                for (size_t i = lo; i < hi; ++i) {
-                    const unsigned long long *q = &h[(size_t)order[i].second * 16 + 8];
-                    for (int j = 0; j < 7; ++j) acc[j] += (double)q[j];
-                    waiting += q[7] == 1 ? 1 : 0;
-                }
-                const double n = (double)std::max<size_t>(hi - lo, 1);
-                fprintf(stderr, "[az_pool profile] last tick, finish %5.1f..%5.1f us (%4zu games): populate %5.1f backup %4.1f descent %5.1f expand %4.1f "
-                                "sum of all %5.1f kcycles | steps %.2f levels %.1f | requested an evaluation %.0f%%\n",
-                        order[lo].first, order[hi - 1].first, hi - lo, acc[0] / n / 1e3, acc[1] / n / 1e3, acc[2] / n / 1e3, acc[3] / n / 1e3,
-                        acc[4] / n / 1e3, acc[5] / n, acc[6] / n, 100.0 * waiting / n);
-            }
-            // the stragglers one by one: the tick ends with the last of them
-            for (size_t i = order.size() > 12 ? order.size() - 12 : 0; i < order.size(); ++i) {
-                const unsigned long long *q = &h[(size_t)order[i].second * 16 + 8];
-                fprintf(stderr, "[az_pool profile] straggler game %5d finished %5.1f us: populate %5.1f backup %4.1f descent %5.1f expand %4.1f "
-                                "all %5.1f kcycles | steps %llu levels %llu status %llu\n",
-                        order[i].second, order[i].first, q[0] / 1e3, q[1] / 1e3, q[2] / 1e3, q[3] / 1e3, q[4] / 1e3, q[5], q[6], q[7]);
-            }
-            if (!finish.empty()) {
-                std::sort(start.begin(), start.end());
-                std::sort(finish.begin(), finish.end());
-                auto pct = [](const std::vector<double> &v, double q) { return v[std::min(v.size() - 1, (size_t)(q * v.size()))]; };
-                fprintf(stderr, "[az_pool profile] last tick, us after the first warp started: starts p50 %.1f p99 %.1f max %.1f | finishes p10 %.1f "
-                                "p50 %.1f p75 %.1f p87 %.1f p95 %.1f p99 %.1f max %.1f\n",
-                        pct(start, 0.5), pct(start, 0.99), start.back(), pct(finish, 0.10), pct(finish, 0.5), pct(finish, 0.75), pct(finish, 0.87),
-                        pct(finish, 0.95), pct(finish, 0.99), finish.back());
-            }
-            cudaFree(grp.dev.prof);
-            grp.dev.prof = nullptr;
+    if (pool->dev.prof) {              // per-phase cycles, accumulated over every tick: mean and worst game
+        std::vector<unsigned long long> h((size_t)pool->dev.G * 16);
+        cudaMemcpy(h.data(), pool->dev.prof, h.size() * 8, cudaMemcpyDeviceToHost);
+        const char *names[6] = {"populate", "backup", "descent", "expand", "make_move", "total"};
+        for (int ph = 0; ph < 6; ++ph) {
+            double sum = 0, mx = 0;
+            for (int g = 0; g < pool->dev.G; ++g) { sum += (double)h[(size_t)g * 16 + ph]; mx = std::max(mx, (double)h[(size_t)g * 16 + ph]); }
+            fprintf(stderr, "[az_pool profile] %-9s mean %.1f kcycles/tick/game, worst game %.1f kcycles/tick (%llu ticks)\n", names[ph],
+                    sum / pool->dev.G / std::max<uint64_t>(pool->ticks, 1) / 1e3, mx / std::max<uint64_t>(pool->ticks, 1) / 1e3,
+                    (unsigned long long)pool->ticks);
         }
-        free_group(grp);
+        // the last tick on the wall clock: when did each game start and finish inside the kernel?
+        std::vector<double> start, finish;
+        unsigned long long t0 = ~0ull;
+        for (int g = 0; g < pool->dev.G; ++g)
+            if (h[(size_t)g * 16 + 6]) t0 = std::min(t0, h[(size_t)g * 16 + 6]);
+        std::vector<std::pair<double, int>> order;
+        for (int g = 0; g < pool->dev.G; ++g)
+            if (h[(size_t)g * 16 + 6]) {
+                start.push_back((double)(h[(size_t)g * 16 + 6] - t0) * 1e-3);
+                finish.push_back((double)(h[(size_t)g * 16 + 7] - t0) * 1e-3);
+                order.push_back({finish.back(), g});
+            }
+        // what the games of each finish-time band did in that tick (cycles per phase, steps, tree levels)
+        std::sort(order.begin(), order.end());
+        const double bands[6] = {0.0, 0.25, 0.5, 0.75, 0.9, 0.97};
+        for (int b = 0; b < 6 && !order.empty(); ++b) {
+            const size_t lo = (size_t)(bands[b] * order.size()), hi = b == 5 ? order.size() : (size_t)(bands[b + 1] * order.size());
+            if (hi <= lo) continue;                    // pools of a few games: not every band has one
+            double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, waiting = 0;
+            for (size_t i = lo; i < hi; ++i) {
+                const unsigned long long *q = &h[(size_t)order[i].second * 16 + 8];
+                for (int j = 0; j < 7; ++j) acc[j] += (double)q[j];
+                waiting += q[7] == 1 ? 1 : 0;
+            }
+            const double n = (double)std::max<size_t>(hi - lo, 1);
+            fprintf(stderr, "[az_pool profile] last tick, finish %5.1f..%5.1f us (%4zu games): populate %5.1f backup %4.1f descent %5.1f expand %4.1f "
+                            "sum of all %5.1f kcycles | steps %.2f levels %.1f | requested an evaluation %.0f%%\n",
+                    order[lo].first, order[hi - 1].first, hi - lo, acc[0] / n / 1e3, acc[1] / n / 1e3, acc[2] / n / 1e3, acc[3] / n / 1e3,
+                    acc[4] / n / 1e3, acc[5] / n, acc[6] / n, 100.0 * waiting / n);
+        }
+        // the stragglers one by one: the tick ends with the last of them
+        for (size_t i = order.size() > 12 ? order.size() - 12 : 0; i < order.size(); ++i) {
+            const unsigned long long *q = &h[(size_t)order[i].second * 16 + 8];
+            fprintf(stderr, "[az_pool profile] straggler game %5d finished %5.1f us: populate %5.1f backup %4.1f descent %5.1f expand %4.1f "
+                            "all %5.1f kcycles | steps %llu levels %llu status %llu\n",
+                    order[i].second, order[i].first, q[0] / 1e3, q[1] / 1e3, q[2] / 1e3, q[3] / 1e3, q[4] / 1e3, q[5], q[6], q[7]);
+        }
+        if (!finish.empty()) {
+            std::sort(start.begin(), start.end());
+            std::sort(finish.begin(), finish.end());
+            auto pct = [](const std::vector<double> &v, double q) { return v[std::min(v.size() - 1, (size_t)(q * v.size()))]; };
+            fprintf(stderr, "[az_pool profile] last tick, us after the first warp started: starts p50 %.1f p99 %.1f max %.1f | finishes p10 %.1f "
+                            "p50 %.1f p75 %.1f p87 %.1f p95 %.1f p99 %.1f max %.1f\n",
+                    pct(start, 0.5), pct(start, 0.99), start.back(), pct(finish, 0.10), pct(finish, 0.5), pct(finish, 0.75), pct(finish, 0.87),
+                    pct(finish, 0.95), pct(finish, 0.99), finish.back());
+        }
+        cudaFree(pool->dev.prof);
+        pool->dev.prof = nullptr;
     }
+    free_buffers(pool);
     delete pool;
 }
 
 extern "C" int az_pool_stats_get(az_pool *pool, az_pool_stats *out)
 {
     AZ_REQUIRE(pool && out, AZ_ERR_ARG, "az_pool_stats_get: null argument");
-    int rc = sync_all(pool);
-    if (rc) return rc;
+    AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
     read_events(pool, 0);                          // every batch has completed: bring the timing sums up to date
     read_events(pool, 1);
     az_pool_stats s{};
-    for (Group &grp : pool->groups) {
-        AZ_CUDA(cudaMemcpy(grp.h_games.data(), grp.dev.games, sizeof(Game) * grp.dev.G, cudaMemcpyDeviceToHost));
-        for (const Game &g : grp.h_games) {
-            s.steps += g.steps;
-            s.evals += g.evals;
-            s.terminal_steps += g.terminal_steps;
-            s.positions += g.positions;
-            s.games_finished += g.finished;
-            s.games_skipped += g.skipped;
-            s.max_depth = std::max<uint64_t>(s.max_depth, g.max_depth);
-            s.levels += g.levels;
-        }
+    AZ_CUDA(cudaMemcpy(pool->h_games.data(), pool->dev.games, sizeof(Game) * pool->dev.G, cudaMemcpyDeviceToHost));
+    for (const Game &g : pool->h_games) {
+        s.steps += g.steps;
+        s.evals += g.evals;
+        s.terminal_steps += g.terminal_steps;
+        s.positions += g.positions;
+        s.games_finished += g.finished;
+        s.games_skipped += g.skipped;
+        s.max_depth = std::max<uint64_t>(s.max_depth, g.max_depth);
+        s.levels += g.levels;
     }
     s.ticks = pool->ticks;
     s.kernel_launches = pool->launches;
@@ -648,12 +556,9 @@ extern "C" int az_pool_stats_get(az_pool *pool, az_pool_stats *out)
     s.tree_seconds = pool->tree_seconds;
     s.tick_seconds = pool->tick_seconds;
     s.timed_ticks = pool->timed_ticks;
-    s.timed_evals = pool->timed_evals_host;
-    for (Group &grp : pool->groups) {
-        unsigned long long n = 0;
-        AZ_CUDA(cudaMemcpy(&n, grp.d_timed_evals, sizeof(n), cudaMemcpyDeviceToHost));
-        s.timed_evals += n;
-    }
+    unsigned long long device_timed_evals = 0;
+    AZ_CUDA(cudaMemcpy(&device_timed_evals, pool->d_timed_evals, sizeof(device_timed_evals), cudaMemcpyDeviceToHost));
+    s.timed_evals = pool->timed_evals_host + device_timed_evals;
     *out = s;
     return AZ_OK;
 }
@@ -664,11 +569,9 @@ extern "C" int az_pool_set_root(az_pool *pool, int game, const az_position *root
     AZ_REQUIRE(game >= 0 && game < pool->G(), AZ_ERR_ARG, "az_pool_set_root: game %d out of range", game);
     AZ_REQUIRE(pool->pending_requests == 0, AZ_ERR_STATE, "az_pool_set_root: evaluations are outstanding (az_pool_provide first)");
     AZ_REQUIRE(valid_position(*root), AZ_ERR_ARG, "az_pool_set_root: invalid position");
-    int local;
-    Group &grp = pool->group_of(game, &local);
-    aztree_launch_set_root(grp.dev, local, *root, grp.stream);
+    aztree_launch_set_root(pool->dev, game, *root, pool->ctx->stream);
     pool->launches++;
-    AZ_CUDA(cudaStreamSynchronize(grp.stream));
+    AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;
 }
@@ -679,14 +582,11 @@ extern "C" int az_pool_set_roots(az_pool *pool, const az_position *roots)
     AZ_REQUIRE(pool->pending_requests == 0, AZ_ERR_STATE, "az_pool_set_roots: evaluations are outstanding (az_pool_provide first)");
     for (int g = 0; g < pool->G(); ++g)
         AZ_REQUIRE(valid_position(roots[g]), AZ_ERR_ARG, "az_pool_set_roots: invalid position for game %d", g);
-    for (Group &grp : pool->groups) {
-        cudaStream_t s = grp.stream;
-        AZ_CUDA(cudaMemcpyAsync(grp.dev.req_pos, roots + grp.first_game, sizeof(az_position) * grp.dev.G, cudaMemcpyHostToDevice, s));
-        aztree_launch_set_roots(grp.dev, grp.dev.req_pos, s);     // req_pos is free between ticks: reuse it as staging
-        pool->launches++;
-    }
-    int rc = sync_all(pool);
-    if (rc) return rc;
+    cudaStream_t s = pool->ctx->stream;
+    AZ_CUDA(cudaMemcpyAsync(pool->dev.req_pos, roots, sizeof(az_position) * pool->dev.G, cudaMemcpyHostToDevice, s));
+    aztree_launch_set_roots(pool->dev, pool->dev.req_pos, s);     // req_pos is free between ticks: reuse it as staging
+    pool->launches++;
+    AZ_CUDA(cudaStreamSynchronize(s));
     AZ_CUDA(cudaGetLastError());
     return check_game_errors(pool);
 }
@@ -696,17 +596,14 @@ extern "C" int az_pool_set_visits(az_pool *pool, int visits)
     AZ_REQUIRE(pool, AZ_ERR_ARG, "az_pool_set_visits: null pool");
     AZ_REQUIRE(visits >= 1 && visits + 2 <= pool->cfg.node_capacity, AZ_ERR_ARG, "az_pool_set_visits: visits=%d does not fit node_capacity=%d",
                visits, pool->cfg.node_capacity);
-    int rc = sync_all(pool);
-    if (rc) return rc;
+    AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
     pool->cfg.visits = visits;
-    for (Group &grp : pool->groups) {
-        grp.dev.visits = visits;
-        // trees that were parked as "done" under the old target may have work again
-        AZ_CUDA(cudaMemcpy(grp.h_games.data(), grp.dev.games, sizeof(Game) * grp.dev.G, cudaMemcpyDeviceToHost));
-        for (Game &g : grp.h_games)
-            if (g.status == ST_DONE) g.status = ST_IDLE;
-        AZ_CUDA(cudaMemcpy(grp.dev.games, grp.h_games.data(), sizeof(Game) * grp.dev.G, cudaMemcpyHostToDevice));
-    }
+    pool->dev.visits = visits;
+    // trees that were parked as "done" under the old target may have work again
+    AZ_CUDA(cudaMemcpy(pool->h_games.data(), pool->dev.games, sizeof(Game) * pool->dev.G, cudaMemcpyDeviceToHost));
+    for (Game &g : pool->h_games)
+        if (g.status == ST_DONE) g.status = ST_IDLE;
+    AZ_CUDA(cudaMemcpy(pool->dev.games, pool->h_games.data(), sizeof(Game) * pool->dev.G, cudaMemcpyHostToDevice));
     return AZ_OK;
 }
 
@@ -722,22 +619,16 @@ extern "C" int az_pool_run(az_pool *pool, int max_ticks, int32_t *idle_out)
     for (int t = 0; t < max_ticks;) {
         const int n = std::min(burst, max_ticks - t);
         for (int k = 0; k < n; ++k) {
-            for (Group &grp : pool->groups) {
-                int rc = launch_tree(pool, grp);
-                if (rc) return rc;
-                if (k == n - 1)
-                    AZ_CUDA(cudaMemcpyAsync(grp.h_counts, grp.dev.req_count + 2 * grp.slot, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, grp.stream));
-                if ((rc = launch_net(pool, grp))) return rc;
-            }
+            int rc = launch_tree(pool);
+            if (rc) return rc;
+            if (k == n - 1)
+                AZ_CUDA(cudaMemcpyAsync(pool->h_counts, pool->dev.req_count + 2 * pool->slot, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, pool->ctx->stream));
+            if ((rc = launch_net(pool))) return rc;
             pool->ticks++;
         }
         t += n;
-        bool idle = true;
-        for (Group &grp : pool->groups) {
-            AZ_CUDA(cudaStreamSynchronize(grp.stream));
-            idle &= grp.h_counts[0] == 0 && grp.h_counts[1] == 0;   // no requests, nobody mid-step: every tree is done (or stalled)
-        }
-        if (idle) {
+        AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
+        if (pool->h_counts[0] == 0 && pool->h_counts[1] == 0) {    // no requests, nobody mid-step: every tree is done (or stalled)
             if (idle_out) *idle_out = 1;
             break;
         }
@@ -752,28 +643,27 @@ extern "C" int az_pool_collect(az_pool *pool, float *features, int32_t *n_reques
     AZ_REQUIRE(pool && features && n_requests, AZ_ERR_ARG, "az_pool_collect: null argument");
     AZ_REQUIRE(pool->cfg.eval_mode == AZ_EVAL_EXTERNAL, AZ_ERR_STATE, "az_pool_collect: pool uses the internal net");
     AZ_REQUIRE(pool->pending_requests == 0, AZ_ERR_STATE, "az_pool_collect: previous requests not answered (az_pool_provide)");
-    Group &grp = pool->groups[0];               // external pools have one group
-    cudaStream_t s = grp.stream;
+    cudaStream_t s = pool->ctx->stream;
     *n_requests = 0;
     // The first tick consumes the evaluations handed in by az_pool_provide.  A tree may burn its step budget
     // on adjudicated leaves without reaching a leaf that needs the net, so "top-up" ticks (which leave the
     // already-waiting games alone and append to the request list) run until no tree can make progress.
     for (int attempt = 0; attempt < 65536; ++attempt) {
-        int rc = launch_tree(pool, grp, attempt == 0);
+        int rc = launch_tree(pool, attempt == 0);
         if (rc) return rc;
         if (attempt == 0) pool->ticks++;
-        AZ_CUDA(cudaMemcpyAsync(grp.h_counts, grp.dev.req_count + 2 * grp.slot, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        AZ_CUDA(cudaMemcpyAsync(pool->h_counts, pool->dev.req_count + 2 * pool->slot, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
         AZ_CUDA(cudaStreamSynchronize(s));
         if ((rc = check_game_errors(pool))) return rc;
         bool busy = false;
-        for (int g = 0; g < grp.dev.G; ++g) busy |= grp.h_games[g].status == ST_IDLE || grp.h_games[g].status == ST_DESCEND;
+        for (int g = 0; g < pool->dev.G; ++g) busy |= pool->h_games[g].status == ST_IDLE || pool->h_games[g].status == ST_DESCEND;
         if (!busy) break;                       // every tree is waiting, done or stalled
     }
-    const int n = std::min(grp.h_counts[0], grp.dev.cap);   // requests beyond the cap stay queued (the tree kernel re-issues them)
+    const int n = std::min(pool->h_counts[0], pool->dev.cap);   // requests beyond the cap stay queued (the tree kernel re-issues them)
     if (n > 0) {
-        aztree_launch_features(grp.dev.req_pos, n, grp.d_features, s);
+        aztree_launch_features(pool->dev.req_pos, n, pool->d_features, s);
         pool->launches++;
-        AZ_CUDA(cudaMemcpyAsync(features, grp.d_features, sizeof(float) * AZ_FEATURES * n, cudaMemcpyDeviceToHost, s));
+        AZ_CUDA(cudaMemcpyAsync(features, pool->d_features, sizeof(float) * AZ_FEATURES * n, cudaMemcpyDeviceToHost, s));
         AZ_CUDA(cudaStreamSynchronize(s));
     }
     AZ_CUDA(cudaGetLastError());
@@ -788,10 +678,9 @@ extern "C" int az_pool_provide_n(az_pool *pool, const float *logits, const float
     AZ_REQUIRE(pool->pending_requests > 0, AZ_ERR_STATE, "az_pool_provide: no outstanding requests");
     const int n = pool->pending_requests;
     AZ_REQUIRE(n_rows == n, AZ_ERR_ARG, "az_pool_provide: %d evaluations handed in for %d outstanding requests", n_rows, n);
-    Group &grp = pool->groups[0];
-    cudaStream_t s = grp.stream;
-    AZ_CUDA(cudaMemcpyAsync(grp.dev.logits, logits, sizeof(float) * AZ_LOGITS * n, cudaMemcpyHostToDevice, s));
-    AZ_CUDA(cudaMemcpyAsync(grp.dev.values, values, sizeof(float) * n, cudaMemcpyHostToDevice, s));
+    cudaStream_t s = pool->ctx->stream;
+    AZ_CUDA(cudaMemcpyAsync(pool->dev.logits, logits, sizeof(float) * AZ_LOGITS * n, cudaMemcpyHostToDevice, s));
+    AZ_CUDA(cudaMemcpyAsync(pool->dev.values, values, sizeof(float) * n, cudaMemcpyHostToDevice, s));
     AZ_CUDA(cudaStreamSynchronize(s));      // the caller may free its arrays right away (complete_workload copies too)
     pool->pending_requests = 0;
     return AZ_OK;
@@ -809,14 +698,12 @@ extern "C" int az_pool_root(az_pool *pool, int game, az_position *pos, int32_t *
 {
     AZ_REQUIRE(pool, AZ_ERR_ARG, "az_pool_root: null pool");
     AZ_REQUIRE(game >= 0 && game < pool->G(), AZ_ERR_ARG, "az_pool_root: game %d out of range", game);
-    int local;
-    Group &grp = pool->group_of(game, &local);
-    AZ_CUDA(cudaStreamSynchronize(grp.stream));
+    AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
     Game gm;
-    AZ_CUDA(cudaMemcpy(&gm, grp.dev.games + local, sizeof(Game), cudaMemcpyDeviceToHost));
+    AZ_CUDA(cudaMemcpy(&gm, pool->dev.games + game, sizeof(Game), cudaMemcpyDeviceToHost));
     AZ_REQUIRE(gm.status != ST_ERROR, AZ_ERR_CAPACITY, "game %d: %s", game, kErrNames[std::min(std::max(gm.error, 0), 3)]);
     std::vector<uint8_t> slot(kNodeStride);
-    AZ_CUDA(cudaMemcpy(slot.data(), grp.dev.nodes + ((size_t)local * grp.dev.C + gm.root) * kNodeStride, kNodeStride,
+    AZ_CUDA(cudaMemcpy(slot.data(), pool->dev.nodes + ((size_t)game * pool->dev.C + gm.root) * kNodeStride, kNodeStride,
                        cudaMemcpyDeviceToHost));
     const NodeHdr *h = reinterpret_cast<const NodeHdr *>(slot.data());
     if (pos) {
@@ -848,15 +735,13 @@ extern "C" int az_pool_pv(az_pool *pool, int game, az_move *moves, int32_t *visi
 {
     AZ_REQUIRE(pool && moves && len_out && max_len >= 0, AZ_ERR_ARG, "az_pool_pv: bad argument");
     AZ_REQUIRE(game >= 0 && game < pool->G(), AZ_ERR_ARG, "az_pool_pv: game %d out of range", game);
-    int local;
-    Group &grp = pool->group_of(game, &local);
-    AZ_CUDA(cudaStreamSynchronize(grp.stream));
+    AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
     Game gm;
-    AZ_CUDA(cudaMemcpy(&gm, grp.dev.games + local, sizeof(Game), cudaMemcpyDeviceToHost));
+    AZ_CUDA(cudaMemcpy(&gm, pool->dev.games + game, sizeof(Game), cudaMemcpyDeviceToHost));
     std::vector<uint8_t> slot(kNodeStride);
     int node = gm.root, n = 0;
     while (n < max_len && node >= 0) {                      // select_principal_variation(best=True), engine.py:331-336
-        AZ_CUDA(cudaMemcpy(slot.data(), grp.dev.nodes + ((size_t)local * grp.dev.C + node) * kNodeStride, kNodeStride, cudaMemcpyDeviceToHost));
+        AZ_CUDA(cudaMemcpy(slot.data(), pool->dev.nodes + ((size_t)game * pool->dev.C + node) * kNodeStride, kNodeStride, cudaMemcpyDeviceToHost));
         const NodeHdr *h = reinterpret_cast<const NodeHdr *>(slot.data());
         const Entry *ent = reinterpret_cast<const Entry *>(slot.data() + kOffEntry);
         int best = -1;
@@ -878,13 +763,11 @@ extern "C" int az_pool_debug_nodes(az_pool *pool, int game, uint64_t *own, uint6
                                    int32_t *n_out)
 {
     AZ_REQUIRE(pool && own && opp && turn && n_out, AZ_ERR_ARG, "az_pool_debug_nodes: bad argument");
-    int local;
-    Group &grp = pool->group_of(game, &local);
-    AZ_CUDA(cudaStreamSynchronize(grp.stream));
+    AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
     Game gm;
-    AZ_CUDA(cudaMemcpy(&gm, grp.dev.games + local, sizeof(Game), cudaMemcpyDeviceToHost));
-    std::vector<uint8_t> arena((size_t)grp.dev.C * kNodeStride);
-    AZ_CUDA(cudaMemcpy(arena.data(), grp.dev.nodes + (size_t)local * grp.dev.C * kNodeStride, arena.size(), cudaMemcpyDeviceToHost));
+    AZ_CUDA(cudaMemcpy(&gm, pool->dev.games + game, sizeof(Game), cudaMemcpyDeviceToHost));
+    std::vector<uint8_t> arena((size_t)pool->dev.C * kNodeStride);
+    AZ_CUDA(cudaMemcpy(arena.data(), pool->dev.nodes + (size_t)game * pool->dev.C * kNodeStride, arena.size(), cudaMemcpyDeviceToHost));
     std::vector<int> queue{gm.root};
     int n = 0;
     for (size_t q = 0; q < queue.size() && n < max_nodes; ++q) {
@@ -905,15 +788,13 @@ extern "C" int az_pool_play(az_pool *pool, int game, az_move move)
     AZ_REQUIRE(pool, AZ_ERR_ARG, "az_pool_play: null pool");
     AZ_REQUIRE(game >= 0 && game < pool->G(), AZ_ERR_ARG, "az_pool_play: game %d out of range", game);
     AZ_REQUIRE(pool->pending_requests == 0, AZ_ERR_STATE, "az_pool_play: evaluations are outstanding");
-    int local;
-    Group &grp = pool->group_of(game, &local);
-    cudaStream_t s = grp.stream;
-    aztree_launch_play(grp.dev, local, (int)move, grp.d_status, s);
+    cudaStream_t s = pool->ctx->stream;
+    aztree_launch_play(pool->dev, game, (int)move, pool->d_status, s);
     pool->launches++;
-    AZ_CUDA(cudaMemcpyAsync(grp.h_counts + 2, grp.d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaMemcpyAsync(pool->h_counts + 2, pool->d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     AZ_CUDA(cudaStreamSynchronize(s));
     AZ_CUDA(cudaGetLastError());
-    const int st = grp.h_counts[2];
+    const int st = pool->h_counts[2];
     AZ_REQUIRE(st != -1, AZ_ERR_ARG, "az_pool_play: move is not legal at the root of game %d", game);
     AZ_REQUIRE(st != -2, AZ_ERR_STATE, "az_pool_play: game %d is waiting for an evaluation", game);
     AZ_REQUIRE(st == 0, AZ_ERR_CAPACITY, "az_pool_play: node pool exhausted");
@@ -922,10 +803,9 @@ extern "C" int az_pool_play(az_pool *pool, int game, az_move move)
 
 namespace {
 
-// `ticks` (<= kTicksPerDrain) iterations of (tree kernel, net kernel) per group, the groups' launches interleaved on their
-// own streams, then one drain of finished games.  Every tick is bracketed by CUDA events on the launching stream; after the
-// drain's synchronisation the per-launch times are summed into tree_seconds / net_seconds / tick_seconds -- every launch is
-// measured, nothing is extrapolated (with several groups these are launch-to-completion times of overlapping kernels).
+// `ticks` (<= kTicksPerDrain) iterations of (tree kernel, net kernel), then one drain of finished games.  Every tick is
+// bracketed by CUDA events on the context stream; after the drain's synchronisation the per-launch times are summed into
+// tree_seconds / net_seconds / tick_seconds -- every launch is measured, nothing is extrapolated.
 //
 // Measured and rejected (r02, profiles/r02_early_launch_trace.txt): launching the net kernel PROGRAMMATICALLY behind the tree
 // kernel (griddepcontrol.launch_dependents + request-slot stamps) so that the tree's tail -- its slowest game takes twice as
@@ -933,23 +813,21 @@ namespace {
 // the tick instead of ~105), but a net CTA can only move onto an SM once most of that SM's games are done, the games still
 // running next to it slow down 1.8x (last finish 173 us instead of 97), and the SMs hosting them start their two CTAs last
 // -- with three 170-us unit passes per CTA nothing can be rebalanced at that granularity, so the kernel ends when it did.
-// read out the event set `set` of every group (its batch has completed) into the pool's timing sums
+// read out the event set `set` (its batch has completed) into the pool's timing sums
 void read_events(az_pool *pool, int set)
 {
-    for (Group &grp : pool->groups) {
-        // ev[0]: before the batch; ev[1 + 2t] / ev[2 + 2t]: behind the tree / the net kernel of tick t.  A kernel's time runs from the
-        // event behind its predecessor, so the launch gap in front of it is part of it.
-        const std::vector<cudaEvent_t> &ev = grp.ev[set];
-        for (int t = 0; t < grp.ev_ticks[set]; ++t) {
-            float a = 0.f, b = 0.f;
-            if (cudaEventElapsedTime(&a, ev[2 * t], ev[2 * t + 1]) != cudaSuccess || cudaEventElapsedTime(&b, ev[2 * t + 1], ev[2 * t + 2]) != cudaSuccess) continue;
-            pool->tree_seconds += a * 1e-3;
-            pool->net_seconds += b * 1e-3;
-            pool->tick_seconds += (a + b) * 1e-3;
-            if (&grp == &pool->groups[0]) pool->timed_ticks++;
-        }
-        grp.ev_ticks[set] = 0;
+    // ev[0]: before the batch; ev[1 + 2t] / ev[2 + 2t]: behind the tree / the net kernel of tick t.  A kernel's time runs from the
+    // event behind its predecessor, so the launch gap in front of it is part of it.
+    const std::vector<cudaEvent_t> &ev = pool->ev[set];
+    for (int t = 0; t < pool->ev_ticks[set]; ++t) {
+        float a = 0.f, b = 0.f;
+        if (cudaEventElapsedTime(&a, ev[2 * t], ev[2 * t + 1]) != cudaSuccess || cudaEventElapsedTime(&b, ev[2 * t + 1], ev[2 * t + 2]) != cudaSuccess) continue;
+        pool->tree_seconds += a * 1e-3;
+        pool->net_seconds += b * 1e-3;
+        pool->tick_seconds += (a + b) * 1e-3;
+        pool->timed_ticks++;
     }
+    pool->ev_ticks[set] = 0;
 }
 
 // everything a caller may look at after an entry point returns: timing sums complete, every record in its file
@@ -964,8 +842,8 @@ int finish_batches(az_pool *pool)
 int run_ticks(az_pool *pool, FILE *out, bool copy_records, int ticks, int64_t *games)
 {
     int rc = AZ_OK;
-    const size_t ng = pool->groups.size();
-    const int set = pool->groups[0].ev_cur;
+    cudaStream_t s = pool->ctx->stream;
+    const int set = pool->ev_cur;
     // Which launches carry events: a timing event between two kernels costs ~3 us of GPU time (the front end cannot prepare
     // the next launch behind it: 0.579 against 0.572 ms per tick with and without them), so the events sit on a CONTIGUOUS
     // window of kEventWindow ticks out of every kEventPeriod -- every tree and net launch inside a window is bracketed, and
@@ -973,34 +851,26 @@ int run_ticks(az_pool *pool, FILE *out, bool copy_records, int ticks, int64_t *g
     // AZ_POOL_EVENT_WINDOW=<ticks> changes the window (>= the period: every tick, 0: none).
     static const int window = getenv("AZ_POOL_EVENT_WINDOW") ? atoi(getenv("AZ_POOL_EVENT_WINDOW")) : kEventWindow;
     const bool timed = (int)(pool->ticks % kEventPeriod) < window;
-    for (size_t gi = 0; gi < ng && timed; ++gi) cudaEventRecord(pool->groups[gi].ev[set][0], pool->groups[gi].stream);
+    if (timed) cudaEventRecord(pool->ev[set][0], s);
     for (int t = 0; t < ticks && rc == AZ_OK; ++t) {
-        for (size_t gi = 0; gi < ng && rc == AZ_OK; ++gi) {
-            Group &grp = pool->groups[gi];
-            grp.dev.timed_evals = (timed && t > 0) ? grp.d_timed_evals : nullptr;      // tick t's tree kernel counts tick t-1's net launch
-            rc = launch_tree(pool, grp);
-            grp.dev.timed_evals = nullptr;
-            if (timed) cudaEventRecord(grp.ev[set][2 * t + 1], grp.stream);
-            if (rc == AZ_OK) rc = launch_net(pool, grp);
-            if (timed) cudaEventRecord(grp.ev[set][2 * t + 2], grp.stream);
-        }
+        pool->dev.timed_evals = (timed && t > 0) ? pool->d_timed_evals : nullptr;      // tick t's tree kernel counts tick t-1's net launch
+        rc = launch_tree(pool);
+        pool->dev.timed_evals = nullptr;
+        if (timed) cudaEventRecord(pool->ev[set][2 * t + 1], s);
+        if (rc == AZ_OK) rc = launch_net(pool);
+        if (timed) cudaEventRecord(pool->ev[set][2 * t + 2], s);
         pool->ticks++;
     }
     if (rc) return rc;
     if (timed)                                    // the batch's last net launch: its request count is read behind the batch
-        for (Group &grp : pool->groups)
-            AZ_CUDA(cudaMemcpyAsync(grp.h_counts + 4, grp.dev.req_count + 2 * grp.slot, sizeof(int32_t), cudaMemcpyDeviceToHost, grp.stream));
-    for (Group &grp : pool->groups) {
-        grp.ev_ticks[set] = timed ? ticks : 0;
-        grp.ev_cur = set ^ 1;
-    }
+        AZ_CUDA(cudaMemcpyAsync(pool->h_counts + 4, pool->dev.req_count + 2 * pool->slot, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    pool->ev_ticks[set] = timed ? ticks : 0;
+    pool->ev_cur = set ^ 1;
     // the previous batch finished before this one was launched: its events are read while the GPU works on this one
     read_events(pool, set ^ 1);
-    for (Group &grp : pool->groups)
-        if ((rc = drain_finished(pool, grp, out, games, copy_records))) return rc;
-    if ((rc = sync_all(pool))) return rc;
-    if (timed)
-        for (Group &grp : pool->groups) pool->timed_evals_host += (uint64_t)std::min(grp.h_counts[4], grp.dev.cap);
+    if ((rc = drain_finished(pool, out, games, copy_records))) return rc;
+    AZ_CUDA(cudaStreamSynchronize(s));
+    if (timed) pool->timed_evals_host += (uint64_t)std::min(pool->h_counts[4], pool->dev.cap);
     return AZ_OK;
 }
 }  // namespace
@@ -1128,7 +998,7 @@ extern "C" void launch_threads(char *output_path, int visits, float *fill_buffer
         cfg.steps_per_tick = 64;
         cfg.seed = g_legacy.ctx->seed + 0x9E3779B97F4A7C15ULL * (h + 1);
         if (az_pool_create(g_legacy.ctx, &cfg, &g_legacy.half[h])) legacy_die("az_pool_create");
-        g_legacy.half[h]->groups[0].dev.cap = buffer_entries;      // a workload is exactly one fill buffer
+        g_legacy.half[h]->dev.cap = buffer_entries;      // a workload is exactly one fill buffer
         g_legacy.waiting[h] = false;
     }
     if (g_legacy.single) { g_legacy.half[1] = g_legacy.half[0]; g_legacy.waiting[1] = false; }
@@ -1155,7 +1025,7 @@ extern "C" int get_workload(void)
     }
     std::memcpy(g_legacy.fill[h], st.data(), sizeof(float) * AZ_FEATURES * (size_t)have);
     int64_t dummy = 0;
-    if (drain_finished(pool, pool->groups[0], g_legacy.out, &dummy) || !pool->writer.flush()) legacy_die("drain");
+    if (drain_finished(pool, g_legacy.out, &dummy) || !pool->writer.flush()) legacy_die("drain");
     g_legacy.waiting[h] = true;
     g_legacy.next ^= 1;
     return h;

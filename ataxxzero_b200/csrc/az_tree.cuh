@@ -144,11 +144,9 @@ struct PoolDev {
     int32_t *done_count;     // [1]
     int32_t G, C, visits, max_plies, noise, auto_play, steps_per_tick;
     int32_t levels_per_tick; // bound on tree levels a game may descend per tick (tail latency of deep endgame lines)
-    int32_t tick_cycles;     // > 0: a game also stops starting new tree levels this many SM clock cycles into the tick
     int32_t cap;             // evaluations served per tick: a whole number of net-kernel rounds; later requests are re-queued
     int32_t consume;         // 1: evaluations of the previous requests are in logits/values; 0: top-up tick, leave waiting games alone
     int32_t tick_slot;       // slot of req_count this tick appends its requests to
-    int32_t game_base;       // global index of this group's game 0 (RNG streams are keyed by the global game index)
     uint32_t rec_cap_words;
     uint64_t seed;
     // speculative evaluation (search pools; all null / 0 otherwise)

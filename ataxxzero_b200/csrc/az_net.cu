@@ -1,5 +1,5 @@
 // az_net.cu -- policy/value network forward pass: weight upload, the fp32 reference-accurate
-// kernel, and the C-ABI entry points.  (The bf16 tcgen05 path lives in az_net_tc.cu.)
+// kernel, and the C-ABI entry points.  (The bf16 / f16 tcgen05 path lives in az_net_pair.cu.)
 //
 // Network (model.py:38-79): conv3x3(4->128)+BN+ReLU; 12 x [conv3x3+BN+ReLU, conv3x3+BN, +skip, ReLU];
 // policy = conv1x1(128->17); value = conv1x1(128->1) -> reshape 49 (x-major) -> fc(49->1)+b -> tanh.
@@ -163,7 +163,7 @@ void az_net_release(az_context *ctx)
 {
     AzNet *n = ctx->net;
     if (!n) return;
-    az_net_tc_release(n);
+    az_net_pair_release(n);
     for (float *p : {n->packed, n->bn_mean, n->bn_scale})
         if (p) cudaFree(p);
     if (n->d_flag) cudaFree(n->d_flag);
@@ -222,7 +222,7 @@ extern "C" int az_net_load(az_context *ctx, const float *packed, size_t count, i
         net->fc_w = p;                      p += 49;
         net->fc_b = p;                      p += 1;
         net->bn_raw = p;
-        int rc = az_net_tc_alloc(net);
+        int rc = az_net_pair_alloc(net);
         if (rc) return rc;
         AZ_CUDA(cudaFuncSetAttribute(k_net_fp32<AZ_IN_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_FP32));
         AZ_CUDA(cudaFuncSetAttribute(k_net_fp32<AZ_IN_POS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_FP32));
@@ -232,7 +232,7 @@ extern "C" int az_net_load(az_context *ctx, const float *packed, size_t count, i
     AZ_CUDA(cudaMemsetAsync(net->d_flag, 0, sizeof(int), s));
     k_prepare_bn<<<(unsigned)((count + 255) / 256), 256, 0, s>>>(net->packed, count, net->bn_raw, net->layers, filters, net->bn_mean,
                                                                  net->bn_scale, net->d_flag);
-    int rc = az_net_tc_prepare(ctx, net);        // bf16 re-tiling with the BN scale folded in, on the device
+    int rc = az_net_pair_prepare(ctx, net);      // bf16 / f16 re-tiling with the BN scale folded in, on the device
     if (rc) return rc;
     ctx->launches += 4;
     int flag = 0;
@@ -247,18 +247,19 @@ extern "C" int az_net_load(az_context *ctx, const float *packed, size_t count, i
 }
 
 static int net_forward_dev(az_context *ctx, const void *d_in, int in_kind, int n, int mode, void *d_logits, void *d_values,
-                           const int *d_count = nullptr, cudaStream_t stream = nullptr, int tiles = 0, double *d_exps = nullptr,
-                           double *d_totals = nullptr, const int *d_out_map = nullptr)
+                           const int *d_count = nullptr, cudaStream_t stream = nullptr, double *d_exps = nullptr, double *d_totals = nullptr,
+                           const int *d_out_map = nullptr, int tiles = 0)
 {
     if (!stream && ctx) stream = ctx->stream;
     AZ_REQUIRE(ctx && (n == 0 || (d_in && (d_logits || d_exps) && d_values)), AZ_ERR_ARG, "az_net_forward: null argument");
     AZ_REQUIRE(ctx->net, AZ_ERR_STATE, "az_net_forward: no weights loaded (call az_net_load first)");
     AZ_REQUIRE(n >= 0, AZ_ERR_ARG, "az_net_forward: n=%d", n);
     AZ_REQUIRE(mode == AZ_NET_FP32 || mode == AZ_NET_BF16 || mode == AZ_NET_F16, AZ_ERR_ARG, "az_net_forward: unknown mode %d", mode);
+    AZ_REQUIRE(!d_out_map || d_exps, AZ_ERR_ARG, "az_net_forward: an output map goes with softmax numerators");
     if (n == 0) return AZ_OK;
     if (mode == AZ_NET_BF16 || mode == AZ_NET_F16)
-        return az_net_tc_forward(ctx, ctx->net, d_in, in_kind, n, static_cast<float *>(d_logits), static_cast<float *>(d_values), d_count, stream, tiles,
-                                 d_exps, d_totals, mode == AZ_NET_F16, d_out_map);
+        return az_net_pair_forward(ctx, ctx->net, d_in, in_kind, n, static_cast<float *>(d_logits), static_cast<float *>(d_values), d_count, stream,
+                                   mode == AZ_NET_F16, d_exps, d_totals, d_out_map, tiles);
     AZ_REQUIRE(!d_exps && !d_out_map, AZ_ERR_ARG, "az_net_forward: softmax numerators are produced by the tensor-core kernel only");
     const int grid = (n + NB - 1) / NB;
     if (in_kind == AZ_IN_F32)
@@ -273,9 +274,9 @@ static int net_forward_dev(az_context *ctx, const void *d_in, int in_kind, int n
 }
 
 int az_net_forward_internal(az_context *ctx, const void *d_in, int in_kind, int n, int mode, float *d_logits, float *d_values,
-                            const int *d_count, cudaStream_t stream, int tiles, double *d_exps, double *d_totals, const int *d_out_map)
+                            const int *d_count, cudaStream_t stream, double *d_exps, double *d_totals, const int *d_out_map)
 {
-    return net_forward_dev(ctx, d_in, in_kind, n, mode, d_logits, d_values, d_count, stream, tiles, d_exps, d_totals, d_out_map);
+    return net_forward_dev(ctx, d_in, in_kind, n, mode, d_logits, d_values, d_count, stream, d_exps, d_totals, d_out_map);
 }
 
 extern "C" int az_net_forward_dev(az_context *ctx, const void *d_features, int n, int mode, void *d_logits, void *d_values)
@@ -294,10 +295,13 @@ extern "C" int az_net_forward_counted_dev(az_context *ctx, const void *d_feature
 // Test hook (not part of the public header): the forward pass exactly as the self-play pool launches it (launch_net in
 // az_pool.cu) -- az_position[] input, board count read from device memory when d_count is non-null, and for a speculative
 // cache pool the softmax numerators, their sequential sums and the values scattered through d_out_map with d_logits null.
+// `tiles` = 1 or 2 forces k_net_pair's tiles per CTA for a plain pass (0: chosen as for the pool); the cache pass has the
+// one-tile schedule only.
 extern "C" int az_net_forward_pool_dev(az_context *ctx, const void *d_pos, int n, const int *d_count, int mode, int tiles, void *d_logits,
                                        void *d_values, double *d_exps, double *d_totals, const int *d_out_map)
 {
-    return net_forward_dev(ctx, d_pos, AZ_IN_POS, n, mode, d_logits, d_values, d_count, nullptr, tiles, d_exps, d_totals, d_out_map);
+    AZ_REQUIRE(tiles >= 0 && tiles <= 2, AZ_ERR_ARG, "az_net_forward_pool_dev: tiles=%d", tiles);
+    return net_forward_dev(ctx, d_pos, AZ_IN_POS, n, mode, d_logits, d_values, d_count, nullptr, d_exps, d_totals, d_out_map, tiles);
 }
 
 extern "C" int az_net_forward_pos_dev(az_context *ctx, const void *d_pos, int n, int mode, void *d_logits, void *d_values)
@@ -382,7 +386,7 @@ extern "C" int az_net_forward_sym8(az_context *ctx, const float *features, int n
     AZ_CUDA(cudaMemcpyAsync(b[0].ptr, features, fb, cudaMemcpyHostToDevice, s));
     if (mode == AZ_NET_BF16 || mode == AZ_NET_F16) {
         // fused: the tensor-core kernel generates the 8 images while it stages its input and averages in its head epilogue
-        int rc = az_net_tc_forward_sym8(ctx, ctx->net, b[0].ptr, AZ_IN_F32, n, b[4].as<float>(), b[5].as<float>(), mode == AZ_NET_F16);
+        int rc = az_net_pair_forward_sym8(ctx, ctx->net, b[0].as<float>(), n, b[4].as<float>(), b[5].as<float>(), mode == AZ_NET_F16);
         if (rc) return rc;
         AZ_CUDA(cudaMemcpyAsync(logits, b[4].ptr, lb, cudaMemcpyDeviceToHost, s));
         AZ_CUDA(cudaMemcpyAsync(values, b[5].ptr, 4 * nn, cudaMemcpyDeviceToHost, s));
@@ -399,6 +403,24 @@ extern "C" int az_net_forward_sym8(az_context *ctx, const float *features, int n
     AZ_CUDA(cudaMemcpyAsync(logits, b[4].ptr, lb, cudaMemcpyDeviceToHost, s));
     AZ_CUDA(cudaMemcpyAsync(values, b[5].ptr, 4 * nn, cudaMemcpyDeviceToHost, s));
     AZ_CUDA(cudaStreamSynchronize(s));
+    AZ_CUDA(cudaGetLastError());
+    return AZ_OK;
+}
+
+// Debug/validation hook (not part of the public header): run the first `conv_layers` convolutions of the
+// tensor-core tower (bf16) and return the fp32 (pre-bf16-rounding) activations [n][49][128] of the last one.
+extern "C" int az_net_debug_tower(az_context *ctx, const float *features, int n, int conv_layers, float *act_out)
+{
+    AZ_REQUIRE(ctx && ctx->net && features && act_out && n > 0, AZ_ERR_ARG, "az_net_debug_tower: bad argument");
+    AZ_REQUIRE(conv_layers >= 1 && conv_layers <= ctx->net->layers, AZ_ERR_ARG, "conv_layers out of range");
+    const size_t fb = sizeof(float) * AZ_FEATURES * (size_t)n, ab = sizeof(float) * 49 * F * (size_t)n;
+    AZ_REQUIRE(ctx->scratch[0].reserve(fb) == 0 && ctx->scratch[1].reserve(ab) == 0, AZ_ERR_CUDA, "scratch alloc");
+    AZ_CUDA(cudaMemcpyAsync(ctx->scratch[0].ptr, features, fb, cudaMemcpyHostToDevice, ctx->stream));
+    AZ_CUDA(cudaMemsetAsync(ctx->scratch[1].ptr, 0, ab, ctx->stream));
+    int rc = az_net_pair_tower(ctx, ctx->net, ctx->scratch[0].as<float>(), n, conv_layers, ctx->scratch[1].as<float>());
+    if (rc) return rc;
+    AZ_CUDA(cudaMemcpyAsync(act_out, ctx->scratch[1].ptr, ab, cudaMemcpyDeviceToHost, ctx->stream));
+    AZ_CUDA(cudaStreamSynchronize(ctx->stream));
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;
 }

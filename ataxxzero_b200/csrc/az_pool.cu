@@ -143,7 +143,7 @@ int launch_net(az_pool *pool)
     int rc;
     if (D.cache_tag)      // speculative search pool: every evaluation of the batch lands in its cache entry
         rc = az_net_forward_internal(pool->ctx, D.req_pos, AZ_IN_POS, D.req_cap, pool->cfg.eval_mode, nullptr, D.cache_val,
-                                     D.req_count + 2 * pool->slot, pool->ctx->stream, 0, D.cache_exps, D.cache_tot, D.req_out);
+                                     D.req_count + 2 * pool->slot, pool->ctx->stream, D.cache_exps, D.cache_tot, D.req_out);
     else
         rc = az_net_forward_internal(pool->ctx, D.req_pos, AZ_IN_POS, D.cap, pool->cfg.eval_mode, D.logits, D.values,
                                      D.req_count + 2 * pool->slot, pool->ctx->stream);
@@ -381,7 +381,7 @@ extern "C" int az_pool_create(az_context *ctx, const az_pool_config *cfg, az_poo
     // request).  AZ_REQ_CAP=<n> sets the cap, 0 serves every request.
     D.cap = D.G;
     if (cfg->auto_play && tensor_net) {
-        const int round = az_net_tc_boards_per_round(ctx);
+        const int round = az_net_pair_boards_per_round(ctx);
         if (const char *env = getenv("AZ_REQ_CAP")) D.cap = atoi(env) > 0 ? std::min(atoi(env), D.G) : D.G;
         else if (D.G >= round) D.cap = D.G / round * round;
     }
@@ -415,7 +415,7 @@ extern "C" int az_pool_create(az_context *ctx, const az_pool_config *cfg, az_poo
         while (entries < 2 * pool->cfg.node_capacity && entries < (1 << 18)) entries *= 2;    // 6.7 KB per entry
         D.cache_entries = entries;
         D.spec_k = spec_k;
-        D.req_cap = std::max(2 * az_net_tc_boards_per_round(ctx), (int)G * (1 + spec_k));
+        D.req_cap = std::max(2 * az_net_pair_boards_per_round(ctx), (int)G * (1 + spec_k));
         const size_t total = G * (size_t)entries + 1;        // + the trash entry
         rc |= dev_alloc(&D.cache_tag, total);
         rc |= dev_alloc(&D.cache_exps, total * AZ_LOGITS, false);

@@ -7,7 +7,7 @@
 //
 // Data layout.  A minibatch of B boards is B*64 GEMM rows: a board is an 8x8 frame whose first row and last column are
 // zero padding (row = 8*(x+1) + y), so a 3x3 tap is a constant row shift and the padding cells double as the conv's zero
-// border between boards (the geometry of az_net_tc.cu).  Two boards form a TILE of 128 rows.  Tensors live in HBM in
+// border between boards (the geometry of az_net_pair.cu).  Two boards form a TILE of 128 rows.  Tensors live in HBM in
 // "tile-blocked" form, which is exactly the shared-memory image the tensor cores read:
 //   TB16 (bf16 operands):  [tile][channel group of 8][row 0..127][8]   32 KiB per tile -- activations, dz
 //   TB32 (fp32 values):    [tile][channel group of 4][row 0..127][4]   64 KiB per tile -- conv outputs z, gradients

@@ -1,5 +1,5 @@
 // az_umma.cuh -- the tcgen05 / mbarrier / bulk-copy PTX wrappers used by az_train.cu (sm_100a).  Internal.
-// (az_net_tc.cu and az_net_pair.cu predate this header and carry their own copies of the ones they use.)
+// (az_net_pair.cu predates this header and carries its own copies of the ones it uses.)
 #pragma once
 #include <cstdint>
 #include <cuda_bf16.h>

@@ -3,11 +3,13 @@
 tests/test_net_gpu.py and tests/test_net_pair_tiles_gpu.py check the plain forward pass from host feature planes.  The search
 runs three other passes of the same kernels, and this file checks each of them against that plain pass, bit for bit, and
 against the fp64 restatement of model.py (oracle/net_numpy.py):
-  * position input: the net encodes az_position[] itself (AZ_IN_POS), under every kernel variant (k_net_pair with one and
-    two tiles, k_net_tc with one and two tiles) and in the three modes, with the board count also read from device memory;
-  * the speculative cache pass: k_net_tc with logits null, the values, the softmax numerators exp((double)logit) and their
-    strictly sequential sums scattered through an output map into a cache table, whose trash row takes dropped requests;
-  * the symmetry ensemble (az_net_forward_sym8): one CTA per position and 4 or 2 passes, several positions per CTA.
+  * position input: the net encodes az_position[] itself (AZ_IN_POS), under both variants of k_net_pair (one and two tiles
+    per CTA) and in the three modes, with the board count also read from device memory;
+  * the speculative cache pass (k_net_pair's one-tile CACHE kind): logits null, the values, the softmax numerators
+    exp((double)logit) and their strictly sequential sums scattered through an output map into a cache table, whose trash
+    row takes dropped requests;
+  * the symmetry ensemble (az_net_forward_sym8, k_net_pair's one-tile SYM8 kind): each CTA evaluates one position at a time
+    in 4 passes of 2 images, several positions per CTA.
 
 S is the device's SM count (148 on a B200) and R = 4 * S a full round of boards: one pass of every CTA of either kernel
 variant.  Sizes around R, 2R and 3R make CTAs walk a second and third unit, and leave partial units at the tail.
@@ -21,11 +23,11 @@ the fp64 oracle takes ~15 ms of host time per board).  At random init they are t
 3e-4 in F16.  At trained scale (oracle.net_numpy.trained_scale_weights, logits of standard deviation 2) they are
 test_bf16_at_trained_scale's: BF16 max 3 % of the largest logit and rms 2.5 % of the logits' deviation, values 0.15; F16
 2e-2; FP32 1e-5 of full scale and 5e-5 on values.  Measured on a B200 (1000 W power limit):
-  * random init, the largest |error| over the sampled boards of every size and variant (the same in all four variants):
+  * random init, the largest |error| over the sampled boards of every size and variant (the same in both variants):
     FP32 logits 1.5e-7, values 1.9e-8; BF16 logits 8.6e-4, values 8.8e-5; F16 logits 9.6e-5, values 1.2e-5.
   * trained scale, position input at R + 1 boards (largest logit 11.1): BF16 logits 0.138 (1.24 % of full scale), rms
     1.38 % of the logits' deviation, values 0.044; F16 logits 1.87e-2, values 9.6e-3; FP32 logits 2.5e-5, values 7.5e-6.
-  * symmetry ensemble, random init (every variant alike): FP32 logits 5.1e-8, values 7.1e-9; BF16 6.0e-4 and 2.9e-5;
+  * symmetry ensemble, random init: FP32 logits 5.1e-8, values 7.1e-9; BF16 6.0e-4 and 2.9e-5;
     F16 5.0e-5 and 3.9e-6.  At trained scale (largest ensemble logit 4.9), BF16: logits 0.093 (1.89 %), rms 0.72 %,
     values 5.0e-3.
 """
@@ -40,12 +42,10 @@ pytestmark = pytest.mark.gpu
 FP32_TOL, BF16_TOL, F16_TOL = 1e-5, 2e-2, 3e-4
 SENTINEL = -7.0
 
-# pair = k_net_pair (the default for plain passes), tc = k_net_tc; the kernel choice is read when weights load
+# k_net_pair with two or one tiles per CTA; the variant is read when weights load
 POS_VARIANTS = {
     "pair2": {"AZ_NET_PAIR_TILES": "2"},
     "pair1": {"AZ_NET_PAIR_TILES": "1"},
-    "tc1": {"AZ_NET_PAIR": "0", "AZ_NET_TILES": "1"},
-    "tc2": {"AZ_NET_PAIR": "0", "AZ_NET_TILES": "2"},
 }
 
 
@@ -321,27 +321,19 @@ def _check_cache_pass(c, arr, planes, n, count, mode, tiles, rng):
     return int(drop[:count].sum())
 
 
-SPEC_RUNS = {
-    "tiles1": ({}, 1, None),
-    "tiles2": ({}, 2, None),
-    "cluster1": ({"AZ_NET_CLUSTER": "1"}, 2, "R+1"),
-    "cluster4": ({"AZ_NET_CLUSTER": "4"}, 1, "2R+3"),
-}
+CACHE_SIZES = ("1", "3", "R-1", "R+1", "2R+3")
 
 
-@pytest.mark.parametrize("run_id", list(SPEC_RUNS))
-def test_speculative_cache_pass(run_id, network, positions, sms):
+@pytest.mark.parametrize("size", CACHE_SIZES)
+def test_speculative_cache_pass(size, network, positions, sms):
     """values, softmax numerators and their sequential totals scattered through out_map: bit for bit the plain pass's values,
     the tree kernel's exp_d of its logits, and the host's in-order float64 sum; rows no live request maps to keep their
     sentinel.  At 2R + 3 boards every CTA sums a second unit in its helper warp while its epilogue runs the next one."""
     from ataxxzero_b200 import net
-    env, tiles, only = SPEC_RUNS[run_id]
     arr, planes = positions
     R = 4 * sms
-    sizes = {"1": 1, "3": 3, "R-1": R - 1, "R+1": R + 1, "2R+3": 2 * R + 3}
-    if only:
-        sizes = {only: sizes[only]}
-    rng = np.random.default_rng(13)
+    n = {"1": 1, "3": 3, "R-1": R - 1, "R+1": R + 1, "2R+3": 2 * R + 3}[size]
+    rng = np.random.default_rng(13 + n)
 
     def run(c):
         import torch
@@ -349,17 +341,16 @@ def test_speculative_cache_pass(run_id, network, positions, sms):
         from ataxxzero_b200 import _native
         net.load_weights(c, network)
         dropped = 0
-        for n in sizes.values():
-            for count in ((n, n - 2) if n > 2 else (n,)):
-                for mode in (net.BF16, net.F16):
-                    dropped += _check_cache_pass(c, arr, planes, n, count, mode, tiles, rng)
-        assert dropped > 0
+        for count in ((n, n - 2) if n > 2 else (n,)):
+            for mode in (net.BF16, net.F16):
+                dropped += _check_cache_pass(c, arr, planes, n, count, mode, 1, rng)
+        assert dropped > 0 or n < 3             # from 3 requests on, one of them always points at the trash row
         d_pos = _device_positions(arr[:4])
         buf = torch.zeros(16 * 833, dtype=torch.float64, device="cuda")
         torch.cuda.synchronize()
         with pytest.raises(az.AzError):          # FP32 has no softmax numerators
-            _native.check(_pool_forward()(c.handle, _dp(d_pos), 4, None, net.FP32, tiles, None, _dp(buf), _dp(buf), _dp(buf), None))
-    _with_env(env, run)
+            _native.check(_pool_forward()(c.handle, _dp(d_pos), 4, None, net.FP32, 1, None, _dp(buf), _dp(buf), _dp(buf), None))
+    _with_env({}, run)
 
 
 def test_speculative_cache_pass_at_trained_scale(trained, positions, sms):
@@ -414,36 +405,34 @@ def _sym8_oracle(nw, planes, idx):
     return want, wv8.mean(axis=1)
 
 
-SYM_RUNS = {"bf16-t%d-c%d" % (t, cs): ("BF16", {"AZ_NET_TILES": str(t), "AZ_NET_CLUSTER": str(cs)})
-            for t in (1, 2) for cs in (1, 2, 4)}
-SYM_RUNS.update({"f16": ("F16", {}), "fp32": ("FP32", {})})
+SYM_SIZES = ("1", "2", "2S-1", "2S+1", "6S+5")
 
 
-@pytest.mark.parametrize("run_id", list(SYM_RUNS))
-def test_symmetry_ensemble(run_id, network, positions, sym_oracle, sms):
-    """az_net_forward_sym8 bit for bit against its definition over the plain pass, at position counts where CTAs evaluate
-    one position (1), one or two (2S - 1, 2S + 1) and up to seven (6S + 5), and within the fp64 bounds of the ensemble mean"""
+@pytest.mark.parametrize("size", SYM_SIZES)
+@pytest.mark.parametrize("mode_name", ("BF16", "F16", "FP32"))
+def test_symmetry_ensemble(mode_name, size, network, positions, sym_oracle, sms):
+    """az_net_forward_sym8 bit for bit against its definition over the plain pass, and within the fp64 bounds of the ensemble
+    mean.  The 2S one-tile CTAs each evaluate one position at a time: one CTA of the only pair has no position (1), both have
+    one (2), the last pair has one CTA without a position (2S - 1), CTAs evaluate one or two (2S + 1) and up to four (6S + 5)."""
     from ataxxzero_b200 import net
-    mode_name, env = SYM_RUNS[run_id]
     mode = getattr(net, mode_name)
+    run_id = "%s-%s" % (mode_name, size)
     arr, planes = positions
-    sizes = (1, 2 * sms - 1, 2 * sms + 1, 6 * sms + 5)
-    ora_idx = {n: np.unique([0, n // 2, n - 1]) for n in sizes}
-    for n in sizes:
-        if n not in sym_oracle:
-            sym_oracle[n] = _sym8_oracle(network, planes, ora_idx[n])
-    want = sym_oracle
+    n = {"1": 1, "2": 2, "2S-1": 2 * sms - 1, "2S+1": 2 * sms + 1, "6S+5": 6 * sms + 5}[size]
+    ora_idx = np.unique([0, n // 2, n - 1])
+    if n not in sym_oracle:
+        sym_oracle[n] = _sym8_oracle(network, planes, ora_idx)
+    want_p, want_v = sym_oracle[n]
     worst = {}
 
     def run(c):
         net.load_weights(c, network)
-        for n in sizes:
-            got_p, got_v = net.evaluate_symmetric(c, planes[:n], mode)
-            ref_p, ref_v = _sym8_reference(c, planes[:n], mode)
-            bad = np.nonzero(~((got_p == ref_p).all(axis=(1, 2, 3)) & (got_v == ref_v)))[0]
-            assert len(bad) == 0, (run_id, n, "positions differing from the reference", bad[:16], len(bad))
-            _within(mode, got_p[ora_idx[n]], got_v[ora_idx[n]], want[n][0], want[n][1], worst)
-    _with_env(env, run)
+        got_p, got_v = net.evaluate_symmetric(c, planes[:n], mode)
+        ref_p, ref_v = _sym8_reference(c, planes[:n], mode)
+        bad = np.nonzero(~((got_p == ref_p).all(axis=(1, 2, 3)) & (got_v == ref_v)))[0]
+        assert len(bad) == 0, (run_id, n, "positions differing from the reference", bad[:16], len(bad))
+        _within(mode, got_p[ora_idx], got_v[ora_idx], want_p, want_v, worst)
+    _with_env({}, run)
     print("symmetry ensemble %s: max |err| vs fp64 (logits, values): %r" % (run_id, worst))
 
 

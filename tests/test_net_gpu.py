@@ -157,26 +157,6 @@ def test_f16_mode_keeps_2e2_at_trained_scale(ctx, nets):
         assert pool.root(0)["root_visits"] >= 40
 
 
-def test_pair_and_single_cta_kernels_agree_bitwise(nets):
-    """k_net_pair (tcgen05 cta_group::2, the default) and k_net_tc (one CTA per tile) consume the same operand images in the same
-    K order with fp32 accumulation: their outputs must be identical bit for bit, in both operand formats"""
-    import os
-    import ataxxzero_b200 as az
-    from ataxxzero_b200 import net
-    feats = _features(77, 31)
-    out = {}
-    for pair in ("1", "0"):
-        os.environ["AZ_NET_PAIR"] = pair          # read when a context first loads weights
-        try:
-            with az.Context(0) as c:
-                net.load_weights(c, nets)
-                out[pair] = [net.forward(c, feats, m) for m in (net.BF16, net.F16)]
-        finally:
-            del os.environ["AZ_NET_PAIR"]
-    for a, b in zip(out["1"], out["0"]):
-        assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
-
-
 def test_modes_agree_and_batch_invariance(ctx, nets):
     from ataxxzero_b200 import net
     feats = _features(64, 9)

@@ -1,6 +1,5 @@
 """The two-tile CTA-pair net kernel (k_net_pair<2>, the default for batches of a full round) against the one-tile kernel
-(k_net_pair<1>) and the single-CTA kernel (k_net_tc): same operand images, same chunk order, fp32 accumulation per tile, so the
-outputs must be identical bit for bit -- at every batch size, with the board count read from device memory as the self-play pool
+(k_net_pair<1>): same operand images, same chunk order, fp32 accumulation per tile, so the outputs must be identical bit for bit -- at every batch size, with the board count read from device memory as the self-play pool
 launches it, and over a whole capped self-play run."""
 import ctypes as C
 import os
@@ -10,7 +9,7 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 
-VARIANTS = ({"AZ_NET_PAIR_TILES": "2"}, {"AZ_NET_PAIR_TILES": "1"}, {"AZ_NET_PAIR": "0"})
+VARIANTS = ({"AZ_NET_PAIR_TILES": "2"}, {"AZ_NET_PAIR_TILES": "1"})
 
 
 def _with_env(env, fn):

@@ -11,7 +11,7 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 KEEP = ("UTC", "UBLKCP", "LDTM", "STTM", "SYNCS", "UCGABAR", "REDUX", "REDG", "ATOMG", "ELECT", "FENCE", "DADD", "DFMA", "DMUL", "MUFU.RCP64H",
         "MUFU.RSQ64H", "LDG", "STG", "ACQBULK", "PREEXIT", "SHFL")
-KERNELS = ("k_net_pair", "k_net_tcILi1ELi1ELi2", "k_tree_tick", "k_walk", "k_samples", "k_convILi2", "k_wgradE")
+KERNELS = ("k_net_pair", "k_tree_tick", "k_walk", "k_samples", "k_convILi2", "k_wgradE")
 
 
 def main():

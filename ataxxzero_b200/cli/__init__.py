@@ -5,4 +5,8 @@
     python -m ataxxzero_b200.cli.looper                       (looper.py)
     python -m ataxxzero_b200.cli.perft                        (perft.py)
     python -m ataxxzero_b200.cli.uai_interface                (uai_interface.py)
+
+and one the reference does not have:
+
+    python -m ataxxzero_b200.cli.arena                        (two networks matched on the GPU)
 """

@@ -54,13 +54,17 @@ def play_one_game(args, engine1, engine2, opening_moves):
 
 
 def write_game_to_pgn(args, path, game, round_index=1):
+    """Appends one game.  A game that starts from a set position carries its FEN ("fen": SetUp / FEN tags), and a game that
+    was not played on the clock its own "time_control" text; games without these keys are written as before."""
     tags = [("Event", "?"), ("Site", "?"), ("Date", datetime.datetime.now().strftime("%Y.%m.%d")), ("Round", "%i" % round_index),
-            ("White", " ".join(game["white"])), ("Black", " ".join(game["black"])),
-            ("Opening", ", ".join(map(uai_encode_move, game["opening"]))),
+            ("White", " ".join(game["white"])), ("Black", " ".join(game["black"]))]
+    if game.get("fen"):
+        tags += [("SetUp", "1"), ("FEN", game["fen"])]
+    tags += [("Opening", ", ".join(map(uai_encode_move, game["opening"]))),
             ("GameStartTime", datetime.datetime.fromtimestamp(game["start_time"]).isoformat()),
             ("GameEndTime", datetime.datetime.fromtimestamp(game["end_time"]).isoformat()),
             ("Plycount", "%i" % len(game["moves"])), ("Result", {1: "1-0", 2: "0-1", "invalid": "1/2-1/2"}[game["result"]]),
-            ("FinalScore", "%i-%i" % game["final_score"]), ("TimeControl", "+%r" % (args.tc,))]
+            ("FinalScore", "%i-%i" % game["final_score"]), ("TimeControl", game.get("time_control") or "+%r" % (args.tc,))]
     with open(path, "a+") as f:
         for key, value in tags:
             print('[%s "%s"]' % (key, value), file=f)

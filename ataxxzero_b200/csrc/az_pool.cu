@@ -1,10 +1,11 @@
 // az_pool.cu -- host runtime of the device-resident game pool: allocation, the tick loop
 // (tree kernel <-> net kernel, no host round trip per evaluation), external-evaluator stepping,
-// reference-format JSON game records, and the legacy 4-function ABI of link.py.
+// reference-format JSON game records, arena pools (two networks playing each other), and the legacy 4-function ABI of link.py.
 //
 // Replaces the thread pool / double-buffered request queue of cpp/self_play_client.cpp:588-749 and
 // the Python feed loop of accelerated_generate_games.py:54-83.
 #include "az_net.h"
+#include "az_rules.cuh"
 #include "az_tree.cuh"
 
 #include <algorithm>
@@ -25,6 +26,7 @@ void aztree_launch_init_all(const PoolDev &P, const az_position &pos, cudaStream
 void aztree_launch_set_root(const PoolDev &P, int g, const az_position &pos, cudaStream_t s);
 void aztree_launch_set_roots(const PoolDev &P, const az_position *d_pos, cudaStream_t s);
 void aztree_launch_play(const PoolDev &P, int g, int move, int *d_status, cudaStream_t s);
+void aztree_launch_arena_start(const PoolDev &P, cudaStream_t s);
 void aztree_launch_release(const PoolDev &P, const DoneEntry *d_done, int n, cudaStream_t s);
 void aztree_launch_features(const az_position *d_pos, int n, float *d_out, cudaStream_t s);
 void aztree_launch_gather(const PoolDev &P, const DoneEntry *d_done, const uint32_t *d_offsets, int n, uint32_t *d_out, cudaStream_t s);
@@ -61,6 +63,7 @@ struct RecordWriter {
 // Every kernel and copy of a pool runs on the context stream.
 struct az_pool {
     az_context *ctx = nullptr;
+    az_context *ctx_b = nullptr;          // arena pools: the context whose network plays for B (trees [S, 2S)); null otherwise
     RecordWriter writer;
     az_pool_config cfg{};
     PoolDev dev{};
@@ -108,7 +111,8 @@ int dev_alloc(T **p, size_t count, bool zero = true)
     return AZ_OK;
 }
 
-const char *kErrNames[] = {"", "node pool exhausted", "selection path longer than 1024 plies", ">= 256 legal moves"};
+const char *kErrNames[] = {"", "node pool exhausted", "selection path longer than 1024 plies", ">= 256 legal moves",
+                           "arena: the partner's move is not legal at this tree's root"};
 
 int check_game_errors(az_pool *pool)
 {
@@ -116,7 +120,7 @@ int check_game_errors(az_pool *pool)
     AZ_CUDA(cudaMemcpy(pool->h_games.data(), pool->dev.games, sizeof(Game) * pool->dev.G, cudaMemcpyDeviceToHost));
     for (int g = 0; g < pool->dev.G; ++g)
         if (pool->h_games[g].status == ST_ERROR)
-            return az_fail(AZ_ERR_CAPACITY, "game %d: %s", g, kErrNames[std::min(std::max(pool->h_games[g].error, 0), 3)]);
+            return az_fail(AZ_ERR_CAPACITY, "game %d: %s", g, kErrNames[std::min(std::max(pool->h_games[g].error, 0), 4)]);
     return AZ_OK;
 }
 
@@ -141,6 +145,16 @@ int launch_net(az_pool *pool)
 {
     const PoolDev &D = pool->dev;
     int rc;
+    if (pool->ctx_b) {    // arena: each player's half of the requests with that player's network, both on the pool's stream
+        const int S = D.G / 2;
+        rc = az_net_forward_internal(pool->ctx, D.req_pos, AZ_IN_POS, D.cap, pool->cfg.eval_mode, D.logits, D.values,
+                                     D.req_count + 2 * pool->slot, pool->ctx->stream);
+        if (rc == AZ_OK)
+            rc = az_net_forward_internal(pool->ctx_b, D.req_pos + S, AZ_IN_POS, D.cap, pool->cfg.eval_mode, D.logits + (size_t)S * AZ_LOGITS,
+                                         D.values + S, D.req_count + 6 + 2 * pool->slot, pool->ctx->stream);
+        pool->launches += 2;
+        return rc;
+    }
     if (D.cache_tag)      // speculative search pool: every evaluation of the batch lands in its cache entry
         rc = az_net_forward_internal(pool->ctx, D.req_pos, AZ_IN_POS, D.req_cap, pool->cfg.eval_mode, nullptr, D.cache_val,
                                      D.req_count + 2 * pool->slot, pool->ctx->stream, D.cache_exps, D.cache_tot, D.req_out);
@@ -312,7 +326,9 @@ void free_buffers(az_pool *pool)
     PoolDev &D = pool->dev;
     void *ptrs[] = {D.nodes, D.games, D.path, D.gstack, D.req_pos, D.req_game, D.req_stage, D.req_mark, D.req_count, D.logits, D.values, D.cache_tag,
                     D.cache_exps, D.cache_tot, D.cache_val, D.req_out, D.records,
-                    D.done, D.done_count, pool->d_done_snapshot, pool->d_status, pool->d_timed_evals, pool->d_features, pool->d_offsets, pool->d_stage};
+                    D.done, D.done_count, pool->d_done_snapshot, pool->d_status, pool->d_timed_evals, pool->d_features, pool->d_offsets, pool->d_stage,
+                    D.arena_slot_game, D.mailbox, const_cast<az_position *>(D.openings), D.arena_moves, D.arena_plies, D.arena_result,
+                    D.arena_counters};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     if (pool->h_counts) cudaFreeHost(pool->h_counts);
@@ -405,7 +421,7 @@ extern "C" int az_pool_create(az_context *ctx, const az_pool_config *cfg, az_poo
     rc |= dev_alloc(&D.req_game, G);
     rc |= dev_alloc(&D.req_stage, G);
     rc |= dev_alloc(&D.req_mark, G);          // zero: no tick 0 is ever launched
-    rc |= dev_alloc(&D.req_count, 8);
+    rc |= dev_alloc(&D.req_count, 12);       // [3][2], and B's [3][2] of an arena pool
     rc |= dev_alloc(&D.logits, G * AZ_LOGITS);
     rc |= dev_alloc(&D.values, G);
     const int spec_k = (tensor_net && !cfg->auto_play) ? std::min(std::max(cfg->speculate, 0), 64) : 0;
@@ -610,6 +626,7 @@ extern "C" int az_pool_set_visits(az_pool *pool, int visits)
 extern "C" int az_pool_run(az_pool *pool, int max_ticks, int32_t *idle_out)
 {
     AZ_REQUIRE(pool, AZ_ERR_ARG, "az_pool_run: null pool");
+    AZ_REQUIRE(!pool->ctx_b, AZ_ERR_STATE, "az_pool_run: arena pools are driven by az_arena_play");
     AZ_REQUIRE(pool->cfg.eval_mode != AZ_EVAL_EXTERNAL, AZ_ERR_STATE, "az_pool_run: pool uses an external evaluator (collect/provide)");
     if (idle_out) *idle_out = 0;
     // Ticks are launched in bursts and the "anything left to do?" counters are read back once per burst: a tick of an
@@ -701,7 +718,7 @@ extern "C" int az_pool_root(az_pool *pool, int game, az_position *pos, int32_t *
     AZ_CUDA(cudaStreamSynchronize(pool->ctx->stream));
     Game gm;
     AZ_CUDA(cudaMemcpy(&gm, pool->dev.games + game, sizeof(Game), cudaMemcpyDeviceToHost));
-    AZ_REQUIRE(gm.status != ST_ERROR, AZ_ERR_CAPACITY, "game %d: %s", game, kErrNames[std::min(std::max(gm.error, 0), 3)]);
+    AZ_REQUIRE(gm.status != ST_ERROR, AZ_ERR_CAPACITY, "game %d: %s", game, kErrNames[std::min(std::max(gm.error, 0), 4)]);
     std::vector<uint8_t> slot(kNodeStride);
     AZ_CUDA(cudaMemcpy(slot.data(), pool->dev.nodes + ((size_t)game * pool->dev.C + gm.root) * kNodeStride, kNodeStride,
                        cudaMemcpyDeviceToHost));
@@ -879,6 +896,7 @@ extern "C" int az_selfplay_run(az_pool *pool, const char *output_path, int64_t t
                                double max_seconds, az_pool_stats *stats_out)
 {
     AZ_REQUIRE(pool, AZ_ERR_ARG, "az_selfplay_run: null pool");
+    AZ_REQUIRE(!pool->ctx_b, AZ_ERR_STATE, "az_selfplay_run: arena pools are driven by az_arena_play");
     AZ_REQUIRE(pool->cfg.auto_play, AZ_ERR_STATE, "az_selfplay_run: pool was created with auto_play = 0");
     AZ_REQUIRE(pool->cfg.eval_mode != AZ_EVAL_EXTERNAL, AZ_ERR_STATE, "az_selfplay_run: external evaluator pools are driven by collect/provide");
     AZ_REQUIRE(target_games > 0 || target_positions > 0 || max_seconds > 0, AZ_ERR_ARG, "az_selfplay_run: no stop condition");
@@ -911,6 +929,7 @@ extern "C" int az_selfplay_run(az_pool *pool, const char *output_path, int64_t t
 extern "C" int az_selfplay_ticks(az_pool *pool, const char *output_path, int64_t ticks, az_pool_stats *stats_out)
 {
     AZ_REQUIRE(pool && ticks >= 0, AZ_ERR_ARG, "az_selfplay_ticks: bad argument");
+    AZ_REQUIRE(!pool->ctx_b, AZ_ERR_STATE, "az_selfplay_ticks: arena pools are driven by az_arena_play");
     AZ_REQUIRE(pool->cfg.auto_play, AZ_ERR_STATE, "az_selfplay_ticks: pool was created with auto_play = 0");
     AZ_REQUIRE(pool->cfg.eval_mode != AZ_EVAL_EXTERNAL, AZ_ERR_STATE, "az_selfplay_ticks: external evaluator pools are driven by collect/provide");
     FILE *out = nullptr;
@@ -929,6 +948,121 @@ extern "C" int az_selfplay_ticks(az_pool *pool, const char *output_path, int64_t
     if (out) fclose(out);
     if (rc) return rc;
     if (frc) return frc;
+    if ((rc = check_game_errors(pool))) return rc;
+    if (stats_out) return az_pool_stats_get(pool, stats_out);
+    return AZ_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// arena: two networks play each other, `slots` games at a time (az_tree.cu, arena_move / arena_receive)
+// ---------------------------------------------------------------------------------------------
+extern "C" int az_arena_create(az_context *ctx_a, az_context *ctx_b, const az_arena_config *cfg, az_pool **out)
+{
+    AZ_REQUIRE(ctx_a && ctx_b && cfg && out, AZ_ERR_ARG, "az_arena_create: null argument");
+    *out = nullptr;
+    AZ_REQUIRE(ctx_a->device == ctx_b->device, AZ_ERR_ARG, "az_arena_create: contexts on devices %d and %d", ctx_a->device, ctx_b->device);
+    AZ_REQUIRE(cfg->slots >= 1 && cfg->slots <= (1 << 19), AZ_ERR_ARG, "az_arena_create: slots=%d", cfg->slots);
+    for (int k = 0; k < 2; ++k)
+        AZ_REQUIRE(cfg->visits[k] >= 1 && cfg->visits[k] <= (1 << 22), AZ_ERR_ARG, "az_arena_create: visits[%d]=%d", k, cfg->visits[k]);
+    AZ_REQUIRE(cfg->eval_mode == AZ_NET_FP32 || cfg->eval_mode == AZ_NET_BF16 || cfg->eval_mode == AZ_NET_F16, AZ_ERR_ARG,
+               "az_arena_create: eval_mode=%d", cfg->eval_mode);
+    AZ_REQUIRE(ctx_a->net && ctx_b->net, AZ_ERR_STATE, "az_arena_create: no weights loaded in context %s (az_net_load)", ctx_a->net ? "b" : "a");
+    az_pool_config pc{};
+    pc.games = 2 * cfg->slots;
+    pc.visits = cfg->visits[0];
+    pc.max_plies = cfg->max_plies;
+    pc.eval_mode = cfg->eval_mode;
+    pc.node_capacity = cfg->node_capacity > 0 ? cfg->node_capacity : std::max(cfg->visits[0], cfg->visits[1]) + 64;
+    az_pool *pool = nullptr;
+    int rc = az_pool_create(ctx_a, &pc, &pool);
+    if (rc) return rc;
+    pool->ctx_b = ctx_b;
+    PoolDev &D = pool->dev;
+    const int S = cfg->slots;
+    D.visits_b = cfg->visits[1];
+    // each half is served in whole net rounds, as a self-play pool is (az_pool_create); both halves hold S trees on one
+    // device, so they share the cap
+    D.cap = S;
+    if (cfg->eval_mode != AZ_NET_FP32) {
+        const int round = az_net_pair_boards_per_round(ctx_a);
+        if (S >= round) D.cap = S / round * round;
+    }
+    rc |= dev_alloc(&D.arena_slot_game, (size_t)S);
+    rc |= dev_alloc(&D.mailbox, (size_t)D.G);
+    rc |= dev_alloc(&D.arena_counters, 4);
+    if (rc) { az_pool_destroy(pool); return rc; }
+    *out = pool;
+    return AZ_OK;
+}
+
+extern "C" int az_arena_play(az_pool *pool, const az_position *openings, int n, az_move *moves, int32_t *plies, int32_t *result,
+                             az_pool_stats *stats_out)
+{
+    AZ_REQUIRE(pool && openings && moves && plies && result, AZ_ERR_ARG, "az_arena_play: null argument");
+    AZ_REQUIRE(pool->ctx_b, AZ_ERR_STATE, "az_arena_play: not an arena pool (az_arena_create)");
+    AZ_REQUIRE(n >= 1 && n <= (1 << 24), AZ_ERR_ARG, "az_arena_play: n=%d", n);
+    std::vector<az_position> start(openings, openings + n);
+    for (int j = 0; j < n; ++j) {
+        AZ_REQUIRE(valid_position(start[j]) && (start[j].turn == 0 || start[j].turn == 1), AZ_ERR_ARG, "az_arena_play: opening %d is invalid", j);
+        AZ_REQUIRE(az::board_result(start[j], nullptr) == 0, AZ_ERR_ARG, "az_arena_play: opening %d is already decided", j);
+        start[j].ply = 0;                         // plies are counted from the opening
+    }
+    PoolDev &D = pool->dev;
+    cudaStream_t s = pool->ctx->stream;
+    const int S = D.G / 2, games = 2 * n, max_plies = D.max_plies;
+    int rc = 0;
+    az_position *d_openings = nullptr;
+    rc |= dev_alloc(&d_openings, (size_t)n, false);
+    D.openings = d_openings;
+    rc |= dev_alloc(&D.arena_moves, (size_t)games * max_plies);
+    rc |= dev_alloc(&D.arena_plies, (size_t)games);
+    rc |= dev_alloc(&D.arena_result, (size_t)games);
+    auto release = [&] {
+        for (void *p : {(void *)d_openings, (void *)D.arena_moves, (void *)D.arena_plies, (void *)D.arena_result})
+            if (p) cudaFree(p);
+        D.openings = nullptr;
+        D.arena_moves = nullptr;
+        D.arena_plies = D.arena_result = nullptr;
+    };
+    if (rc) { release(); return rc; }
+    D.arena_games = games;
+    const int32_t counters[4] = {std::min(S, games), 0, 0, 0};
+    cudaError_t e = cudaMemcpyAsync(d_openings, start.data(), sizeof(az_position) * n, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(D.arena_counters, counters, sizeof(counters), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = cudaMemsetAsync(D.mailbox, 0, sizeof(uint4) * D.G, s);
+    if (e == cudaSuccess) {
+        aztree_launch_arena_start(D, s);
+        pool->launches++;
+        e = cudaGetLastError();
+    }
+    // Ticks run in bursts (as in az_pool_run) and the finished-game counter is read once per burst.  A game lasts at most
+    // max_plies moves of at most max(visits) evaluations each, and a request waits at most S / cap ticks for the net: the
+    // bound on ticks only stops a pool that cannot make progress.
+    const int64_t games_per_slot = (games + S - 1) / S;
+    const int64_t max_ticks = 4 * games_per_slot * max_plies * (int64_t)(std::max(D.visits, D.visits_b) + 2) * ((S + D.cap - 1) / D.cap);
+    int64_t ticks = 0;
+    int burst = 1;
+    while (e == cudaSuccess && rc == AZ_OK) {
+        for (int k = 0; k < burst && rc == AZ_OK; ++k) {
+            rc = launch_tree(pool);
+            if (rc == AZ_OK) rc = launch_net(pool);
+            pool->ticks++;
+        }
+        ticks += burst;
+        if (rc) break;
+        e = cudaMemcpyAsync(pool->h_counts, D.arena_counters, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess || pool->h_counts[1] >= games || pool->h_counts[2] > 0) break;
+        if (ticks >= max_ticks) { rc = az_fail(AZ_ERR_STATE, "az_arena_play: %d of %d games finished after %lld ticks", pool->h_counts[1], games, (long long)ticks); break; }
+        burst = std::min(2 * burst, 16);
+    }
+    if (e == cudaSuccess && rc == AZ_OK) e = cudaMemcpyAsync(moves, D.arena_moves, sizeof(az_move) * games * max_plies, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess && rc == AZ_OK) e = cudaMemcpyAsync(plies, D.arena_plies, sizeof(int32_t) * games, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess && rc == AZ_OK) e = cudaMemcpyAsync(result, D.arena_result, sizeof(int32_t) * games, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    release();
+    if (e != cudaSuccess) return az_fail(AZ_ERR_CUDA, "az_arena_play: %s", cudaGetErrorString(e));
+    if (rc) return rc;
     if ((rc = check_game_errors(pool))) return rc;
     if (stats_out) return az_pool_stats_get(pool, stats_out);
     return AZ_OK;

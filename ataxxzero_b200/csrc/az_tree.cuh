@@ -53,8 +53,9 @@ enum : uint32_t {
     NF_RANKED = 4u,      // rank[] is valid for the node's current population
     NF_REPOPULATED = 8u  // the node became a root: the reference re-inserted its posterior into a clear()ed map (:489-490)
 };
-enum : int32_t { ST_IDLE = 0, ST_WAIT = 1, ST_DONE = 2, ST_STALL = 3, ST_ERROR = 4, ST_DESCEND = 5 };
-enum : int32_t { ERR_NODES = 1, ERR_PATH = 2, ERR_MOVES = 3 };
+enum : int32_t { ST_IDLE = 0, ST_WAIT = 1, ST_DONE = 2, ST_STALL = 3, ST_ERROR = 4, ST_DESCEND = 5,
+                 ST_PARK = 6 };  // arena: the partner tree's player is to move; this tree waits for its move in the mailbox
+enum : int32_t { ERR_NODES = 1, ERR_PATH = 2, ERR_MOVES = 3, ERR_MAIL = 4 };
 
 struct __align__(16) NodeHdr {
     uint64_t own, opp;       // pieces of the side to move / of the opponent
@@ -137,6 +138,7 @@ struct PoolDev {
     int32_t *req_count;      // [3 slots][2]: {requests, games that still have work but made no request} of a tick.  Ticks
                              // rotate through the slots (tick_slot); a tick reads its predecessor's request count (of which
                              // the first `cap` were evaluated) and zeroes its successor's slot, so the host never memsets.
+                             // Arena pools: player B's half has its own [3][2] at req_count + 6.
     float *logits;           // [G][833]
     float *values;           // [G]
     uint32_t *records;       // [G][2][rec_cap_words]
@@ -165,6 +167,19 @@ struct PoolDev {
     int32_t force_slow;      // test knob (AZ_TREE_FORCE_SLOW=1): resolve every candidate by the full scan
     unsigned long long *timed_evals;   // non-null: the previous tick's net launch was event-timed -- add the evaluations it served
     unsigned long long *prof;   // AZ_POOL_PROFILE=1: [G][8] clock cycles per phase of the last tick (debug aid, normally nullptr)
+    // arena pools (az_arena_create; all null / 0 otherwise): G = 2S trees, [0, S) play for A, [S, 2S) for B, slot s pairs tree s
+    // with tree s + S.  Each half orders its requests on its own (k_order_requests, one block per half) into req_pos[half * S ...]
+    // and is evaluated by its own network; `cap` applies to each half.
+    int32_t *arena_slot_game;   // [S] game index slot s plays; -1: no game left
+    uint4 *mailbox;             // [G] posts to a tree from its partner: {tick of a game-over post, 0, tick of a move post, move};
+                                // a post is read from the tick after the one that stamped it, and cleared by the reader
+    const az_position *openings;// [n] game i starts from openings[i >> 1]; A moves first when i is even
+    uint16_t *arena_moves;      // [2n][max_plies] the moves of every game
+    int32_t *arena_plies;       // [2n]
+    int32_t *arena_result;      // [2n] 1 x won, 2 o won, 0 max_plies reached
+    int32_t *arena_counters;    // [0] next game index, [1] games finished, [2] trees that hit an error
+    int32_t arena_games;        // 2n
+    int32_t visits_b;           // visit target of B's trees (A's: visits)
 };
 
 }  // namespace aztree

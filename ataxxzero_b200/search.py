@@ -1,7 +1,8 @@
 """Device-resident PUCT search / self-play pools over the C ABI.
 
 Mirrors the C++ reference's search objects (cpp/self_play_client.cpp:369-493 ``MCTS``:
-ctor / ``step`` / ``play``; :508-582 ``generate_game``) for G concurrent games at once.
+ctor / ``step`` / ``play``; :508-582 ``generate_game``) for G concurrent games at once, and the arena
+(``Arena``, ``random_openings``) that plays two networks against each other with the same trees.
 """
 import ctypes as C
 
@@ -188,3 +189,93 @@ class Pool:
         stats = PoolStats()
         check(lib().az_pool_stats_get(self._h, C.byref(stats)))
         return stats.as_dict()
+
+
+class ArenaConfig(C.Structure):
+    _fields_ = [("slots", C.c_int32), ("visits", C.c_int32 * 2), ("max_plies", C.c_int32), ("eval_mode", C.c_int32),
+                ("node_capacity", C.c_int32), ("reserved", C.c_int32 * 2)]
+
+
+_native.register("az_arena_create", C.c_int, [_vp, _vp, C.POINTER(ArenaConfig), C.POINTER(_vp)])
+_native.register("az_arena_play", C.c_int, [_vp, _vp, C.c_int, _vp, _vp, _vp, C.POINTER(PoolStats)])
+
+
+class Arena:
+    """Network A (loaded in ``ctx_a``) against network B (``ctx_b``, may be ``ctx_a``) on the GPU, ``slots`` games at a time.
+    Every opening is played twice, A moving first in the even game and B in the odd one; each move is the most visited root
+    edge of the mover's search (no noise, no sampling)."""
+
+    def __init__(self, ctx_a, ctx_b, slots, visits_a, visits_b, eval_mode=EVAL_BF16, max_plies=400, node_capacity=0):
+        cfg = ArenaConfig()
+        cfg.slots, cfg.max_plies, cfg.eval_mode, cfg.node_capacity = int(slots), int(max_plies), int(eval_mode), int(node_capacity)
+        cfg.visits[0], cfg.visits[1] = int(visits_a), int(visits_b)
+        self.cfg = cfg
+        self.max_plies = int(max_plies) if int(max_plies) > 0 else 400
+        self._h = _vp()
+        check(lib().az_arena_create(ctx_a.handle, ctx_b.handle, C.byref(cfg), C.byref(self._h)))
+        ctx_a.adopt(self)
+        if ctx_b is not ctx_a:
+            ctx_b.adopt(self)
+
+    def close(self):
+        if self._h:
+            lib().az_pool_destroy(self._h)
+            self._h = _vp()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def play(self, openings):
+        """Plays the 2n games of n openings.  Returns a dict of per-game arrays: ``moves`` (list of move lists), ``plies``,
+        ``result`` (1 x won, 2 o won, 0 max_plies reached), ``a_is_x`` (True where network A had x), plus ``stats``."""
+        from .rules import positions_array
+        arr = positions_array(openings)
+        n = len(arr)
+        moves = np.zeros((max(2 * n, 1), self.max_plies), dtype=np.uint16)
+        plies = np.zeros(max(2 * n, 1), dtype=np.int32)
+        result = np.zeros(max(2 * n, 1), dtype=np.int32)
+        stats = PoolStats()
+        check(lib().az_arena_play(self._h, C.c_void_p(arr.ctypes.data), n, C.c_void_p(moves.ctypes.data),
+                                  C.c_void_p(plies.ctypes.data), C.c_void_p(result.ctypes.data), C.byref(stats)))
+        games = np.arange(2 * n)
+        a_first = games % 2 == 0
+        x_first = arr["turn"][games >> 1] == 0
+        return {"moves": [[unpack_move(m) for m in moves[i, :plies[i]]] for i in range(2 * n)], "plies": plies[:2 * n].copy(),
+                "result": result[:2 * n].copy(), "a_is_x": a_first == x_first, "stats": stats.as_dict()}
+
+
+def random_openings(ctx, n, plies, seed=0, start_fen=None):
+    """``n`` distinct positions reached after ``plies`` uniformly random plies from ``start_fen`` (default: the self-play start
+    with its four blockers), none of them decided, played on the device (rules.random_playouts).  A repeated opening would
+    repeat its games exactly, so the positions are distinct.  Raises ValueError when random play does not reach n of them."""
+    from .rules import START_FEN, positions_array, random_playouts, set_board
+    start = set_board(start_fen or START_FEN)
+    if plies == 0:
+        if n != 1:
+            raise ValueError("only one distinct opening after 0 plies")
+        start.ply = 0
+        return positions_array([start])
+    out, seen = [], set()
+    batch = max(2 * n, 64)
+    for attempt in range(8):
+        recs, n_plies, _ = random_playouts(ctx, start, batch, max_plies=plies + 1, seed=(int(seed) << 8) + attempt)
+        for g in np.flatnonzero(n_plies > plies):        # a move was played from the position after `plies`: not decided
+            r = recs[g, plies]
+            key = (int(r["x"]), int(r["o"]))
+            if key in seen:
+                continue
+            seen.add(key)
+            out.append((0, (start.turn + plies) & 1, start.blockers, key))
+            if len(out) == n:
+                return np.array(out, dtype=positions_array([]).dtype)
+        batch *= 2
+    raise ValueError("random play reached only %d distinct undecided positions after %d plies, %d asked for" % (len(out), plies, n))

@@ -219,6 +219,30 @@ int az_selfplay_run(az_pool *pool, const char *output_path, int64_t target_games
  * output_path = NULL finished games are recycled on the device and their records are not copied out. */
 int az_selfplay_ticks(az_pool *pool, const char *output_path, int64_t ticks, az_pool_stats *stats_out);
 
+/* ---------------- arena: two networks play each other on the device ------------------ */
+/* An arena pool holds 2*slots search trees: trees [0, slots) search for player A, trees [slots, 2*slots) for player B, and slot s
+ * plays one game at a time between tree s and tree s + slots.  Only the tree whose player is to move searches (no noise, no
+ * sampling); at its player's visit target it plays the most visited root edge (first created on equal counts: az_pool_pv,
+ * engine.py:331-336 best=True) and both trees re-root on the move (az_pool_play).  A free slot takes the next game index. */
+typedef struct {
+    int32_t slots;          /* concurrent games; the pool holds 2*slots trees                                       */
+    int32_t visits[2];      /* visit target per move of player A / player B (1 .. 2^22)                              */
+    int32_t max_plies;      /* a game ends with result 0 when its ply count (from the opening) reaches it; 0 = 400   */
+    int32_t eval_mode;      /* AZ_NET_FP32 / AZ_NET_BF16 / AZ_NET_F16, both players                                  */
+    int32_t node_capacity;  /* nodes per tree; 0 = max(visits) + 64                                                  */
+    int32_t reserved[2];
+} az_arena_config;
+/* Player A is evaluated with the network loaded in ctx_a, player B with the one in ctx_b (same device; ctx_b may be
+ * ctx_a).  Every kernel runs on ctx_a's stream.  az_pool_destroy and az_pool_stats_get work on the pool; az_pool_run and
+ * az_selfplay_* refuse it (AZ_ERR_STATE). */
+int az_arena_create(az_context *ctx_a, az_context *ctx_b, const az_arena_config *cfg, az_pool **out);
+/* Plays the 2*n games of n openings (host az_position[n], none already decided) to the end: game i starts from opening i >> 1,
+ * A moves first in the even games and B in the odd ones.  Outputs are host arrays indexed by game: moves [2n][max_plies]
+ * (az_move; the first plies[i] entries of row i are the game, the rest 0), plies [2n], result [2n] (1 x won, 2 o won, 0
+ * max_plies reached).  stats_out may be NULL.  AZ_ERR_STATE on a pool that az_arena_create did not make. */
+int az_arena_play(az_pool *pool, const az_position *openings, int n, az_move *moves, int32_t *plies, int32_t *result,
+                  az_pool_stats *stats_out);
+
 /* ---------------- training-sample extraction (train.py:43-77 get_sample_from_entries) ---------------- */
 /* A minibatch of (features, policy target, value target) triples straight from ply records.
  *   plies:   table of ply records, uint32 words each: [0,1] x bitboard, [2,3] o bitboard, [4] played move | entries<<16,
